@@ -41,7 +41,9 @@ LOSS_LAG = 8   # e2e leg: the host consumes step k's loss while step k + LOSS_LA
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=48)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps: train steps (default 48), GridEncoder fwd / fwd+bwd "
+                    "iterations of --config encoder (default 12), frames of --config infer (default --frames, the orbit is "
+                    "cycled), CPU steps of --impl reference (default 12)")
     ap.add_argument("--warmup", type=int, default=8)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="train", choices=["train", "infer", "encoder"], help="train: the -O train step (the headline "
@@ -81,15 +83,25 @@ def parse():
     ap.add_argument("--no-shading", action="store_true", help="skip the secondary lambertian-vs-albedo step timing")
     ap.add_argument("--ref-steps", type=int, default=200, help="timed steps of the reference CUDA-extension pipeline")
     ap.add_argument("--ref-warmup", type=int, default=50)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="after the timed steps, write what the last timed step "
+                    "returned as DIR/<name>.npy in float32 / float64, to compare two builds output for output: train: its loss "
+                    "and the model state it left; infer: the last frame's rgb and depth; encoder: a fixed sample of the last "
+                    "backward's table gradient; --impl reference: its loss and the model state")
+    args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 12 if (args.impl == "reference" or args.config == "encoder") else (
+            args.frames if args.config == "infer" else 48)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------
 # reference arm / cpu baseline: the reference's pure-PyTorch non-cuda-ray renderer on host cores
 # ---------------------------------------------------------------------------------------------------
-def cpu_reference_run(steps, warmup):
+def cpu_reference_run(steps, warmup, dump_dir=None):
     """BASELINE.json configs[0]: 64x64 rays x (64+32) samples, vanilla NeRF, fp32 fwd+bwd on CPU.
-    Returns (samples/s, ms/step, cores, description)."""
+    Returns (samples/s, ms/step, cores, description); dump_dir: write the last step's results (dump_outputs)."""
     import torch
     from oracle import torch_renderer as TR
     # all host cores, whatever the launcher exported (torchrun sets OMP_NUM_THREADS=1 for every rank)
@@ -104,9 +116,11 @@ def cpu_reference_run(steps, warmup):
     t0 = time.perf_counter()
     n = 0
     for i in range(steps):
-        k, _ = TR.train_step(model, *views[i % 4], G)
+        k, res = TR.train_step(model, *views[i % 4], G)
         n += k
     dt = time.perf_counter() - t0
+    if dump_dir:
+        dump_outputs(dump_dir, {k: v for k, v in res.items() if torch.is_tensor(v)})
     cores = torch.get_num_threads()
     desc = ("%d fwd+bwd steps of one 64x64-ray view x (64+32) samples through a port of nerf/renderer.py:run + "
             "nerf/network.py (fp32, %d torch threads of %d host cpus)" % (steps, cores, os.cpu_count() or 0))
@@ -117,9 +131,9 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 12))
+    steps = args.steps
     warm = max(1, min(args.warmup, 2))
-    v, ms, cores, desc = cpu_reference_run(steps, warm)
+    v, ms, cores, desc = cpu_reference_run(steps, warm, dump_dir=args.dump_outputs)
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
         "warmup": warm, "ms_per_step": ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
@@ -189,6 +203,27 @@ def build_model(device):
     model = NeRFNetwork(opt).to(device)
     model.train()
     return model
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: {name: tensor} as out_dir/<name>.npy; floating tensors as float32, integer ones as float64 (exact).
+    Nothing is written when the whole exceeds DUMP_LIMIT_BYTES."""
+    import numpy as np
+    import torch
+    conv = {}
+    for name, t in arrays.items():
+        if t is not None:
+            t = torch.as_tensor(t).detach().cpu()
+            conv[name] = (t.float() if t.is_floating_point() else t.double()).numpy()
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes, more than %d" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in conv.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measure_l2_peaks(device):
@@ -290,6 +325,7 @@ def run_b200_arm(args):
     sample_acc = step_fn.samples
 
     step_events = []
+    last_loss = [None]
 
     def run_steps(n, e2e, start_index, record=False):
         for s in range(n):
@@ -300,6 +336,7 @@ def run_b200_arm(args):
             i = start_index + s
             # graph mode copies the packed batch straight into the step's static input buffer (H2D when it is a host batch)
             loss = step_fn(host_batch(i) if e2e else dev_pool[i % n_pool])
+            last_loss[0] = loss
             if e2e:
                 # device -> host read of the step's result, every step: the loss is copied to pinned host memory right
                 # behind the step and consumed LOSS_LAG calls later (TrainStep.read_loss_async), --sync-loss: loss.item().
@@ -353,6 +390,9 @@ def run_b200_arm(args):
     ms_e2e = f0.elapsed_time(f1)
     samples_e2e = int(sample_acc.item())
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # before the untimed profiling steps below, which train the model further
+        dump_outputs(args.dump_outputs, dict(model.state_dict(), loss=last_loss[0]))   # ~17 MB
 
     if args.kernel_table and rank == 0:
         from torch.profiler import profile, ProfilerActivity
@@ -764,7 +804,7 @@ def run_infer_config(args):
     device = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
     torch.cuda.set_device(device)
     _cabi.load()
-    R, n_frames = args.res, args.frames
+    R, n_frames, n_timed = args.res, args.frames, args.steps
     model = build_model(device)
     with torch.autocast("cuda", torch.float16):
         model.update_extra_state()       # the random-init scene: the density blob, ~5.6 % of the grid occupied
@@ -794,7 +834,7 @@ def run_infer_config(args):
     launches0 = _cabi.LAUNCHES
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for i in range(n_frames):
+    for i in range(n_timed):
         frame(i, False)
     e1.record()
     torch.cuda.synchronize()
@@ -802,11 +842,13 @@ def run_infer_config(args):
     launches = _cabi.LAUNCHES - launches0
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     f0.record()
-    for i in range(n_frames):
+    for i in range(n_timed):
         frame(i, True)
     f1.record()
     torch.cuda.synchronize()
     ms_e2e = f0.elapsed_time(f1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"rgb": rgb_host, "depth": depth_host})   # the last timed frame, as read back
     clk = clocks.stop()
     # loop shape + samples of a few frames (diagnostics, untimed): iterations of the device loop, and the per-kernel times
     # of the same frames through the host loop (CUDA events around the entry points)
@@ -834,19 +876,19 @@ def run_infer_config(args):
     gathers_s, _ = measure_l2_peaks(device)
     dom = max(kern, key=lambda k: kern[k][0]) if kern else None
     line = {
-        "metric": "NeRF inference frames/s (800x800, 100-frame orbit, march_rays/composite_rays)", "value": n_frames / (ms * 1e-3),
-        "unit": "frames/s", "n_gpus": 1, "steps": n_frames, "warmup": max(args.warmup, 3), "ms_per_step": ms / n_frames,
+        "metric": "NeRF inference frames/s (800x800, 100-frame orbit, march_rays/composite_rays)", "value": n_timed / (ms * 1e-3),
+        "unit": "frames/s", "n_gpus": 1, "steps": n_timed, "warmup": max(args.warmup, 3), "ms_per_step": ms / n_timed,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f16", "data": "synthetic",
         "config": {"workload": "BASELINE configs[4]: inference render %dx%d via march_rays / composite_rays with the occupancy "
                                "grid, %d-frame 360-degree orbit (circle poses r 1.8, theta 60, fov 55), random-init scene "
                                "(density blob), max_steps 1024, T_thresh 1e-4, white background" % (R, R, n_frames),
-                   "rays_per_frame": R * R, "rays_per_s": R * R * n_frames / (ms * 1e-3),
+                   "rays_per_frame": R * R, "rays_per_s": R * R * n_timed / (ms * 1e-3),
                    "inference_loop": type(model).infer_loop + " (one cudaGraphLaunch per frame, conditional WHILE node)",
                    "loop_iterations_per_frame": iters, "host_loop_ms_per_frame": host_loop_ms,
                    "timing": "every frame renders a different camera; a frame's sample / accumulator buffers (>60 MB) are "
                              "rewritten every loop iteration"},
-        "e2e": {"value": n_frames / (ms_e2e * 1e-3), "unit": "frames/s", "h2d_bytes_per_step": 64,
-                "d2h_bytes_per_step": R * R * 16, "ms_per_step": ms_e2e / n_frames},
+        "e2e": {"value": n_timed / (ms_e2e * 1e-3), "unit": "frames/s", "h2d_bytes_per_step": 64,
+                "d2h_bytes_per_step": R * R * 16, "ms_per_step": ms_e2e / n_timed},
         "gpu_launches": launches, "clocks": clk,
         "roofline": {"kernel": dom, "bound": "l2-gather" if dom == "ngp_field_forward" else "latency", "unit": "GB/s",
                      "achieved": None, "peak": gathers_s * 4 / 1e9, "frac": None, "traffic": None,
@@ -865,7 +907,7 @@ def run_infer_config(args):
             tag = [l for l in out.stdout.splitlines() if l.startswith("REF_PIPELINE_JSON ")]
             line["ref_cuda_ext"] = json.loads(tag[-1][len("REF_PIPELINE_JSON "):]) if tag else {"unavailable": (out.stderr or out.stdout)[-300:]}
             if "ms_per_frame_median" in line["ref_cuda_ext"]:
-                line["ref_cuda_ext"]["speedup_e2e_vs_ref_median"] = line["ref_cuda_ext"]["ms_per_frame_median"] / (ms_e2e / n_frames)
+                line["ref_cuda_ext"]["speedup_e2e_vs_ref_median"] = line["ref_cuda_ext"]["ms_per_frame_median"] / (ms_e2e / n_timed)
         except Exception as e:  # noqa: BLE001
             line["ref_cuda_ext"] = {"unavailable": repr(e)[:200]}
     emit(line)
@@ -922,7 +964,7 @@ def run_encoder_config(args):
     clocks = ClockSampler(device.index)
     clocks.start()
     time.sleep(1.0)
-    steps, warm = max(args.steps // 4, 8), max(args.warmup, 3)
+    steps, warm = args.steps, max(args.warmup, 3)
     launches0 = _cabi.LAUNCHES
     t_f = timed(fwd, steps, warm)
     t_fb = timed(fwd_bwd, steps, warm)
@@ -933,6 +975,11 @@ def run_encoder_config(args):
         enc.embeddings.grad.view(-1)[:1].cpu()          # a read of the step's result
     t_e2e = timed(e2e, steps, warm)
     clk = clocks.stop()
+    if args.dump_outputs:
+        # the table gradient of the last timed fwd + bwd (67 MB in fp32): a fixed sample of 2^20 of its rows
+        rows = np.sort(np.random.default_rng(0).choice(enc.embeddings.shape[0], 1 << 20, replace=False))
+        dump_outputs(args.dump_outputs, {"embeddings_grad_rows": torch.from_numpy(rows),
+                                         "embeddings_grad_sample": enc.embeddings.grad[torch.from_numpy(rows).to(device)]})
     gathers_s, reds_s = measure_l2_peaks(device)
     peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json"))) if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")) else {}
     ach = 512.0 * B / (t_f * 1e-3) / 1e9

@@ -19,10 +19,10 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = "/root/reference"
 sys.path.insert(0, ROOT)
 
 from oracle import torch_renderer as TR  # noqa: E402
+from oracle.build_ref import REF  # noqa: E402  (the reference's source tree, NGP_REFERENCE_ROOT)
 
 
 def import_reference():

@@ -224,11 +224,13 @@ int oracle_grid_encode_forward(const float* inputs, const void* embeddings, cons
 
 /* kernel_grid_backward, gridencoder.cu:227-313.  The reference scatters with order-nondeterministic
  * atomics (fp16 table under autocast); the oracle accumulates the same per-corner addends
- * (w * grad, rounded to half first iff round_addend_to_half) into a DOUBLE table = the exact sum. */
+ * (w * grad, rounded to half first iff round_addend_to_half) into a DOUBLE table = the exact sum
+ * (accumulate 0), or, like the reference's atomics in sample order, rounds the running sum to
+ * float (accumulate 1) or half (accumulate 2) after every add. */
 int oracle_grid_encode_backward(const void* grad, const float* inputs, const int* offsets, double* grad_table,
                                 uint32_t B, uint32_t D, uint32_t C, uint32_t L, float S, uint32_t H,
                                 uint32_t gridtype, int align_corners, int dtype, int grad_layout,
-                                int round_addend_to_half, const float* scale_override) {
+                                int round_addend_to_half, int accumulate, const float* scale_override) {
     if (D < 1 || D > 5 || C > 8) return -2;
     float* scales = (float*)malloc(sizeof(float) * L);
     uint32_t* ress = (uint32_t*)malloc(sizeof(uint32_t) * L);
@@ -265,7 +267,10 @@ int oracle_grid_encode_backward(const void* grad, const float* inputs, const int
                 for (uint32_t c = 0; c < C; ++c) {
                     float v = w * load_elem(grad, go + c, dtype);
                     if (round_addend_to_half) v = round_h(v); /* :302 */
-                    grad_table[tbl + row * C + c] += (double)v;
+                    double* t = grad_table + tbl + row * C + c;
+                    if (accumulate == 1)      *t = (double)((float)*t + v);
+                    else if (accumulate == 2) *t = (double)round_h((float)*t + v);
+                    else                      *t += (double)v;
                 }
             }
         }

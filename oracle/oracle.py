@@ -73,8 +73,9 @@ def grid_encode_forward(inputs, embeddings, offsets, S, H, calc_dydx=False, grid
 
 
 def grid_encode_backward(grad, inputs, offsets, n_rows, Cc, S, H, gridtype=0, align_corners=False, grad_layout=BLC,
-                         round_addend_to_half=False, scale_override=None):
-    """kernel_grid_backward (gridencoder.cu:227-313) with exact (float64) accumulation.
+                         round_addend_to_half=False, scale_override=None, accumulate="exact"):
+    """kernel_grid_backward (gridencoder.cu:227-313) with exact (float64) accumulation, or with the running sum rounded
+    to float32 / float16 after every add in sample order (accumulate "f32" / "f16", like the reference's atomics).
     Returns grad_embeddings float64 [n_rows, C]."""
     inputs = _c(inputs, np.float32)
     offsets = _c(offsets, np.int32)
@@ -87,7 +88,8 @@ def grid_encode_backward(grad, inputs, offsets, n_rows, Cc, S, H, gridtype=0, al
     rc = lib().oracle_grid_encode_backward(_p(grad), _p(inputs), _p(offsets), _p(table), C.c_uint32(B), C.c_uint32(D),
                                            C.c_uint32(Cc), C.c_uint32(L), C.c_float(S), C.c_uint32(H),
                                            C.c_uint32(gridtype), C.c_int(int(align_corners)), C.c_int(dt),
-                                           C.c_int(grad_layout), C.c_int(int(round_addend_to_half)), _p(so))
+                                           C.c_int(grad_layout), C.c_int(int(round_addend_to_half)),
+                                           C.c_int(("exact", "f32", "f16").index(accumulate)), _p(so))
     if rc != 0:
         raise RuntimeError("oracle_grid_encode_backward rc=%d" % rc)
     return table

@@ -14,6 +14,13 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
 
 
+def pytest_report_header(config):
+    from oracle import ref_ext as r
+    built = all(os.path.exists(os.path.join(r.REF_DIR, n + ".so")) for n in ("_gridencoder", "_raymarching", "_freqencoder"))
+    return "ref_ext tests compare against: " + ("the reference's own CUDA extensions (oracle/_ref)" if built else
+                                                "the C oracle stand-in (oracle/ref_standin.py; oracle/_ref is not built)")
+
+
 def pytest_collection_modifyitems(config, items):
     try:
         import torch
@@ -30,9 +37,8 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def ref_ext():
-    """The reference's own CUDA extensions (oracle/_ref), or skip when they were not built."""
+    """The reference's own CUDA extensions (oracle/_ref) when they were built, else the C oracle behind the same calls
+    (oracle/ref_standin.py), which test_golden.py pins to stored outputs of those extensions."""
     from oracle import ref_ext as r
-    mods = r.load()
-    if mods is None:
-        pytest.skip("oracle/_ref extensions not available")
-    return mods
+    from oracle import ref_standin
+    return r.load() or ref_standin.load()

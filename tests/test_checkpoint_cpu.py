@@ -99,16 +99,18 @@ def test_state_dict_matches_the_real_reference_models_manifest():
 
 
 def test_cross_load_with_the_real_reference_model():
-    """With /root/reference present (this container; not the GPU box): build the REAL reference model, load its
+    """With the reference's source tree present (NGP_REFERENCE_ROOT): build the REAL reference model, load its
     state_dict into ours and ours into it with strict=True, and round-trip a reference-Trainer-shaped checkpoint file."""
     import pytest
-    if not os.path.isdir("/root/reference/nerf") or not os.path.isdir(os.path.join(ROOT, "oracle", "_ref")):
+    from oracle.build_ref import REF
+    if not os.path.isdir(os.path.join(REF, "nerf")) or not os.path.isdir(os.path.join(ROOT, "oracle", "_ref")):
         pytest.skip("the reference tree / its built extension modules are not available here")
     import subprocess
     code = r'''
 import argparse, os, sys, tempfile, torch
 ROOT = %r
 sys.path.insert(0, ROOT)
+from oracle.build_ref import REF
 from oracle.make_golden_host import import_reference_grid_model
 RefNet, _, _ = import_reference_grid_model()
 opt = argparse.Namespace(bound=1, cuda_ray=True, min_near=0.1, density_thresh=10, bg_radius=1.4)
@@ -120,7 +122,7 @@ ref_sd = {k: v.clone() for k, v in ref.state_dict().items()}
 # the product package shadows the reference's top-level module names: import it in a clean module table
 for name in [n for n in sys.modules if n.split(".")[0] in ("gridencoder", "raymarching", "freqencoder", "encoding", "activation", "nerf")]:
     del sys.modules[name]
-sys.path = [p for p in sys.path if not p.startswith("/root/reference") and not p.endswith("oracle/_ref")]
+sys.path = [p for p in sys.path if not p.startswith(REF) and not p.endswith("oracle/_ref")]
 sys.path.insert(0, os.path.join(ROOT, "single-stable-dreamfusion_b200"))
 from ngp_b200.network_grid import NeRFNetwork
 from ngp_b200 import checkpoint as ck

@@ -10,7 +10,7 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+from oracle.build_ref import REF  # noqa: E402  (the reference's source tree, NGP_REFERENCE_ROOT)
 
 CODE = r'''
 import argparse, importlib, inspect, os, sys, types

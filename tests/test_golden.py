@@ -99,7 +99,40 @@ def test_oracle_morton_freq_vs_reference_golden():
     assert np.abs(gi - GOLD["freq_gin"]).max() < 1e-4 * np.abs(GOLD["freq_gin"]).max()
 
 
+@pytest.mark.parametrize("dt", ["f32", "f16"])
+@pytest.mark.parametrize("gridtype", [0, 1])
+def test_reference_standin_grid_vs_reference_golden(gridtype, dt):
+    """The stand-in the GPU tests use when the reference's extensions are not built, through the reference's calling
+    convention: forward bit-exact, table gradient accumulated in the table's dtype within the reference's own spread."""
+    import torch
+    from oracle import ref_ext as R
+    from oracle import ref_standin
+    ns = ref_standin.load()
+    c = util.golden_grid_case(gridtype, dt)
+    key = "grid_g%d_%s_" % (gridtype, dt)
+    T = torch.from_numpy
+    out, dydx, _ = R.grid_encode_forward(ns, T(c["x"]), T(c["emb"]), T(c["offs"]), float(c["S"]), c["H"], True, gridtype, False)
+    assert np.array_equal(out.numpy(), GOLD[key + "out"]) and np.array_equal(dydx.numpy(), GOLD[key + "dydx"])
+    ge, gi = R.grid_encode_backward(ns, T(c["grad"]), T(c["x"]), T(c["emb"]), T(c["offs"]), float(c["S"]), c["H"], dydx, gridtype,
+                                    False)
+    assert ge.dtype == T(c["emb"]).dtype
+    rows = np.random.default_rng(5).integers(0, ge.shape[0], 4096)
+    assert util.rel_l2(ge.double().numpy()[rows], GOLD[key + "gemb_rows"]) < (1e-5 if dt == "f32" else 3e-3)
+    assert np.array_equal(gi.numpy(), GOLD[key + "ginp"].astype(gi.numpy().dtype))
+
+
 # ------------------------------------------------------------------------------------------------ GPU
+@pytest.mark.gpu
+def test_reference_standin_freq_kernel_vs_reference_golden():
+    """oracle/ref_freq.cu, the stand-in's fast-math frequency encoder, is bit-exact with the reference's stored output."""
+    import torch
+    from oracle import ref_standin
+    fx = np.random.default_rng(42).uniform(-1, 1, (128, 3)).astype(np.float32)
+    out = torch.empty(128, 39, device="cuda:0")
+    ref_standin.load().freq.freq_encode_forward(torch.from_numpy(fx).to("cuda:0"), 128, 3, 6, 39, out)
+    assert np.array_equal(out.cpu().numpy(), GOLD["freq_out"])
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("dt", ["f32", "f16"])
 @pytest.mark.parametrize("gridtype", [0, 1])

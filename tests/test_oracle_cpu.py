@@ -18,6 +18,30 @@ def test_half_conversion_matches_numpy():
     assert np.array_equal(got.view(np.uint16), want.view(np.uint16))
 
 
+@pytest.mark.parametrize("dtype,accumulate", [(np.float32, "exact"), (np.float32, "f32"), (np.float16, "f16")])
+def test_grid_backward_accumulation_modes(dtype, accumulate):
+    """Every sample at x = 0 of a 1-D level: corner weights 0.5 / 0.5 (exact), so rows 0 and 1 receive the same addends in
+    sample order.  Each mode must equal the numpy sum it names: float64, float32 rounded after every add, or float16 rounded
+    after every add of the half-rounded addend (the reference's fp16 atomics)."""
+    B = 4096
+    g = (np.random.default_rng(3).standard_normal((B, 1)) * 4).astype(dtype)
+    x = np.zeros((B, 1), np.float32)
+    offs = np.array([0, 24], np.int32)
+    table = O.grid_encode_backward(g, x, offs, 24, 1, 1.0, 16, gridtype=1, round_addend_to_half=dtype == np.float16,
+                                   accumulate=accumulate)
+    add = (np.float32(0.5) * g[:, 0].astype(np.float32)).astype(dtype)
+    if accumulate == "exact":
+        want = add.astype(np.float64).sum()
+    else:
+        acc = dtype(0)
+        for v in add:
+            acc = dtype(np.float32(acc) + np.float32(v))
+        want = float(acc)
+    assert np.count_nonzero(table) == 2 and table[0, 0] == want and table[1, 0] == want
+    if accumulate != "exact":
+        assert want != add.astype(np.float64).sum()     # the case tells the modes apart
+
+
 def test_morton_known_answers_and_roundtrip():
     coords = np.array([[0, 0, 0], [1, 0, 0], [0, 1, 0], [0, 0, 1], [1, 1, 1], [127, 127, 127], [5, 3, 9], [1023, 0, 1023]],
                       np.int32)
