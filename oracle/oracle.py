@@ -425,6 +425,60 @@ def bg_backward(fwd, d_rgb):
     return g
 
 
+def adam_scaler_step(p, g, m, v, state, seg_end, seg_lr, betas=(0.9, 0.99), eps=1e-15, grad_div=1.0, lr_decay_ln=0.0,
+                     lr_decay_steps=0.0, growth=2.0, backoff=0.5, growth_interval=2000):
+    """TEST INFRASTRUCTURE - float64 restatement of ONE ``ngp_adam_step`` launch after its finite check (optim.py
+    FusedAdamScaler.step; csrc/train_step.cu adam_step_kernel), i.e. ``scaler.step(optimizer); scaler.update();
+    optimizer.zero_grad()`` on torch.optim.Adam + LambdaLR + GradScaler over one flat buffer:
+
+      found_inf = state[3] or any non-finite g  ->  p, m, v untouched; scale *= backoff, tracker = 0, skipped += 1
+      else  g / (scale * grad_div) -> m.lerp_(g, 1 - b1), v = b2 v + (1 - b2) g^2,
+            p -= lr_seg * exp(lr_decay_ln * min(step, lr_decay_steps)) / (1 - b1^t) * m / (sqrt(v) / sqrt(1 - b2^t) + eps)
+            with t = step + 1; step = t; tracker += 1, scale *= growth (if finite) once tracker reaches growth_interval
+      the gradients come back zeroed either way.
+
+    p, g, m, v: flat float arrays of one length; state: [scale, growth tracker, steps, found_inf, skipped, ...] (optim.py
+    FusedAdamScaler.state); seg_end: exclusive end of each lr group; seg_lr: its lr.  The scalar arguments are narrowed to
+    float32 first, as the launch receives them.  Returns (p, g, m, v, state) as new float64 arrays."""
+    f32 = lambda x: float(np.float32(x))  # noqa: E731
+    b1, b2, eps = f32(betas[0]), f32(betas[1]), f32(eps)
+    p = np.array(p, np.float64)
+    m = np.array(m, np.float64)
+    v = np.array(v, np.float64)
+    g = np.asarray(g)
+    st = np.array(state, np.float64)
+    scale, tracker, steps = st[0], st[1], st[2]
+    skip = st[3] != 0 or not np.isfinite(g).all()
+    if skip:
+        st[0], st[1], st[4] = scale * f32(backoff), 0.0, st[4] + 1
+    else:
+        t = steps + 1
+        bc1, bc2_sqrt = 1.0 - b1 ** t, np.sqrt(1.0 - b2 ** t)
+        lr_mult = np.exp(f32(lr_decay_ln) * min(steps, f32(lr_decay_steps))) if lr_decay_ln != 0 else 1.0
+        lr = np.empty_like(p)
+        start = 0
+        for end, seg in zip(seg_end, seg_lr):
+            lr[start:int(end)] = f32(seg)
+            start = int(end)
+        if start != p.size:
+            raise ValueError("seg_end must end at the buffer's length")
+        gr = np.asarray(g, np.float64) / (scale * f32(grad_div))
+        m += (1.0 - b1) * (gr - m)
+        v *= b2
+        v += (1.0 - b2) * gr * gr
+        denom = np.sqrt(v) / bc2_sqrt + eps
+        p -= lr * (lr_mult / bc1) * m / denom
+        tracker += 1
+        if tracker >= growth_interval:
+            grown = scale * f32(growth)
+            if np.isfinite(np.float32(grown)):
+                scale = grown
+            tracker = 0.0
+        st[0], st[1], st[2] = scale, tracker, t
+    st[3] = 0.0
+    return p, np.zeros(g.shape, np.float64), m, v, st
+
+
 def get_rays(poses, intrinsics, H, W):
     """TEST INFRASTRUCTURE - numpy restatement of nerf/utils.py:43-106 get_rays for the full image (N = -1): pixel centres
     at +0.5 (:60-61), directions ((i - cx) / fx, (j - cy) / fy, 1) (:93-96) normalised by safe_normalize (:33-36, clamp of

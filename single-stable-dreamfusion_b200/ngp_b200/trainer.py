@@ -1002,6 +1002,10 @@ class TrainStep:
                     dst.copy_(src)
                 o.state[5].copy_(torch.maximum(err, o.state[5]))
                 o.flat_grads.zero_()
+                if self._g_table_odd is not None:
+                    # the odd-row twin of the table gradient: pipelined mode leaves the last warm-up step's share there
+                    # (its update, which folds it, is still pending) - it would land in the first real update
+                    self._g_table_odd.zero_()
                 # (o._sync - the cross-GPU barrier epoch - keeps counting: the peers' flags carry it)
             else:
                 for p, q in zip(self.model.parameters(), snap["params"]):

@@ -25,13 +25,14 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REPORT = {}
 
 
-def _report(key, value):
-    REPORT[key] = value
+def _report(key, value, report=REPORT, name="step_parity.json"):
+    """Record `value` under `key` in `report` and rewrite the report file `name` in the output directory."""
+    report[key] = value
     try:
         out = os.path.join(ROOT, "gpurun_out")
         os.makedirs(out, exist_ok=True)
-        with open(os.path.join(out, "step_parity.json"), "w") as f:
-            json.dump(REPORT, f, indent=1, sort_keys=True)
+        with open(os.path.join(out, name), "w") as f:
+            json.dump(report, f, indent=1, sort_keys=True)
     except OSError:
         pass
 

@@ -481,3 +481,67 @@ def test_field_and_bg_oracle_gradients_match_finite_differences():
     fd = (bg_loss(W1p, b2) - bg_loss(W1m, b2)) / 2e-5
     # (gb is evaluated at the fp16-rounded activations; the un-rounded graph agrees to fp16 noise)
     assert abs(fd - gb["w1"][5, 7]) <= 2e-2 * abs(gb["w1"][5, 7]) + 1e-4, (fd, gb["w1"][5, 7])
+
+
+def test_adam_scaler_step_matches_torch_adam_gradscaler_lambdalr():
+    """oracle.adam_scaler_step (the float64 checker of the Adam + GradScaler launch) against torch.optim.Adam +
+    torch.amp.GradScaler + LambdaLR on the CPU: two lr groups split inside a float4 (boundary not a multiple of 4), a
+    gradient divisor, an inf step and a NaN step (skipped: scale backs off, moments untouched), growth every 3 steps and
+    an lr decay that saturates before the end."""
+    torch = pytest.importorskip("torch")
+    rng = np.random.default_rng(0)
+    shapes = [(1001, 2), (64, 32), (64,), (3,)]
+    params = [torch.nn.Parameter(torch.from_numpy((rng.standard_normal(s) * 0.1).astype(np.float32))) for s in shapes]
+    n0 = params[0].numel()
+    assert n0 % 4 != 0
+    lrs, iters, grad_div, interval = (1e-2, 1e-3), 5, 2.0, 3
+    opt = torch.optim.Adam([{"params": params[:1], "lr": lrs[0]}, {"params": params[1:], "lr": lrs[1]}], betas=(0.9, 0.99),
+                           eps=1e-15)
+    sched = torch.optim.lr_scheduler.LambdaLR(opt, lambda it: 0.1 ** min(it / iters, 1))
+    scaler = torch.amp.GradScaler("cpu", growth_interval=interval)
+    scaler.scale(torch.zeros(1))                    # GradScaler creates its scale lazily
+    flat = lambda ts: np.concatenate([t.detach().numpy().reshape(-1) for t in ts]).astype(np.float64)  # noqa: E731
+    p = flat(params)
+    m, v = np.zeros_like(p), np.zeros_like(p)
+    state = np.array([65536.0, 0, 0, 0, 0, 0, 0, 0])
+    seg_end = [n0, p.size]
+    scales = []
+    for it in range(12):
+        raw = [(rng.standard_normal(s) * 10.0 ** (it % 4 - 3)).astype(np.float32) for s in shapes]
+        if it == 4:
+            raw[2][7] = np.inf
+        if it == 9:
+            raw[0][3, 1] = np.nan
+        scale = scaler.get_scale()
+        assert scale == state[0], (it, scale, state[0])
+        scales.append(scale)
+        for q, r in zip(params, raw):
+            q.grad = torch.from_numpy(r * np.float32(scale))
+        g = flat([q.grad for q in params]) * grad_div   # e.g. the sum over 2 data-parallel ranks, divided by the launch
+        if it:                                      # teacher forcing: every step starts from torch's fp32 state
+            st = [opt.state[q] for q in params]
+            p, m, v = flat(params), flat([s["exp_avg"] for s in st]), flat([s["exp_avg_sq"] for s in st])
+        before = dict(p=p, m=m, v=v)
+        scaler.step(opt)
+        scaler.update()
+        if it not in (4, 9):
+            sched.step()                            # once per successful iteration, as the Trainer does
+        p, g_out, m, v, state = O.adam_scaler_step(p, g, m, v, state, seg_end, lrs, grad_div=grad_div,
+                                                   lr_decay_ln=np.log(0.1) / iters, lr_decay_steps=iters,
+                                                   growth_interval=interval)
+        assert not g_out.any() and state[3] == 0
+        if it in (4, 9):
+            assert all(np.array_equal(a, before[k]) for k, a in (("p", p), ("m", m), ("v", v)))
+        st = [opt.state[q] for q in params]
+        for k, want, got in (("p", p, flat(params)), ("m", m, flat([s["exp_avg"] for s in st])),
+                             ("v", v, flat([s["exp_avg_sq"] for s in st]))):
+            # fp32 torch against float64: relative to the value and to this step's change of it (moments cross zero)
+            err = np.abs(got - want) / (np.abs(want) + np.abs(want - before[k]) + 1e-30)
+            assert err.max() < 2e-5, (it, k, float(err.max()))
+        assert int(state[2]) == int(st[0]["step"]) == it + 1 - (it >= 4) - (it >= 9)
+        assert state[1] == float(scaler._growth_tracker)
+    assert state[4] == 2 and state[0] == scaler.get_scale()
+    # the scale grew, backed off on each skipped step and grew again
+    assert scales[3] == 2 * scales[0] and scales[5] == scales[4] / 2 and scales[9] > scales[5] and scales[10] == scales[9] / 2
+    # the decay saturated: the lr stopped shrinking after `iters` successful steps
+    assert opt.param_groups[0]["lr"] == pytest.approx(lrs[0] * 0.1)
