@@ -302,17 +302,21 @@ int ngp_bg_backward(const float* dirs, const float* grad_rgb, uint32_t N, const 
                     const void* b2, uint32_t degree, uint32_t hidden, float* gw1, float* gb1, float* gw2, float* gb2,
                     void* stream);
 
-/* The optimisation step as ONE cooperative launch, with the data-parallel gradient all-reduce fused in over NVLink
- * peer memory (csrc/dp_step.cu): replaces ngp_check_finite + ngp_adam_step (world == 1) and, for world > 1, the
- * all_reduce DistributedDataParallel would issue for the reference's dormant wrap (nerf/utils.py:200-202) as well.
+/* ngp_adam_step for world > 1 ranks with the data-parallel gradient all-reduce fused in over NVLink peer memory
+ * (csrc/adam.cu): the all_reduce DistributedDataParallel would issue for the reference's dormant wrap
+ * (nerf/utils.py:200-202) and the update in one plain launch of independent blocks (block b owns sub-slice b of its
+ * rank's slice: flag exchange - P2P / multimem reduce - Adam - parameter broadcast - flag exchange - clear).  The
+ * GradScaler verdict comes from each rank's OWN bucket: the caller runs ngp_check_finite(grads, n, state + 3) on the same
+ * stream first (a sum of <= 8 finite fp32 gradients is finite), and it travels with the first flag exchange.  Arguments as
+ * ngp_adam_step, and:
  *   state f32[8]: as ngp_adam_step, plus [5] = 1 if a cross-GPU wait timed out (sticky: from then on the step is a no-op
  *   on every rank that saw the flag - nothing is reduced, updated, broadcast or cleared).  sync u32[2], zero-initialised:
- *   [0] block election, [1] barrier epoch.  n must be a multiple of 4.
- *   world > 1: peer_* are HOST arrays of `world` device addresses (this rank's own buffers included, in rank order) of
- *   every rank's gradient bucket, parameter buffer, fp16 shadow and flag pad (ngp_dp_flags_bytes() bytes, zeroed once),
- *   all mapped into this process (symmetric memory / CUDA IPC).  Each rank reduces and updates slice `rank` and writes
- *   the new parameters to every replica; exp_avg / exp_avg_sq are maintained for that slice only.  The gradient bucket
- *   is zero-filled on the way out.  All ranks must launch the same sequence of calls.
+ *   [0] block election, [1] barrier epoch.  n must be a multiple of 4, 2 <= world <= NGP_DP_MAX_WORLD.
+ *   peer_* are HOST arrays of `world` device addresses (this rank's own buffers included, in rank order) of every rank's
+ *   gradient bucket, parameter buffer, fp16 shadow (may be NULL without half_shadow) and flag pad (ngp_dp_flags_bytes()
+ *   bytes, zeroed once), all mapped into this process (symmetric memory / CUDA IPC).  Each rank reduces and updates slice
+ *   `rank` and writes the new parameters to every replica; exp_avg / exp_avg_sq are maintained for that slice only.  The
+ *   gradient bucket is always zero-filled on the way out.  All ranks must launch the same sequence of calls.
  *   multicast: NULL, or a HOST array of 3 NVLS multicast addresses of the gradient bucket, the parameters and the shadow
  *   (the same symmetric allocation mapped through the NVSwitch): the reduce-scatter then is one multimem.ld_reduce per
  *   element (summed inside the switch) and the parameter broadcast one multimem.st instead of `world` P2P stores.
@@ -321,18 +325,6 @@ int ngp_bg_backward(const float* dirs, const float* grad_rgb, uint32_t N, const 
  *   time"); the caller clears state[6] after flushing the last pending update. */
 #define NGP_DP_MAX_WORLD 8
 #define NGP_DP_MAX_BLOCKS 256
-int ngp_adam_step_fused(float* params, float* grads, float* exp_avg, float* exp_avg_sq, void* half_shadow, uint64_t n,
-                        uint32_t n_segments, const uint64_t* seg_end, const float* seg_lr, float beta1, float beta2,
-                        float eps, float grad_div, float lr_decay_ln, float lr_decay_steps, float growth_factor,
-                        float backoff_factor, uint32_t growth_interval, int deferred, float* state, uint32_t* sync,
-                        uint32_t rank, uint32_t world, const uint64_t* peer_grads, const uint64_t* peer_params, const uint64_t* peer_half,
-                        const uint64_t* peer_flags, const uint64_t* multicast, void* stream);
-/* world > 1, second generation: the same data-parallel step WITHOUT grid-wide barriers, as a plain launch of independent
- * blocks (block b owns sub-slice b of its rank's slice: flag exchange - P2P / multimem reduce - Adam - parameter broadcast -
- * flag exchange - clear).  The GradScaler verdict comes from each rank's OWN bucket (the caller runs ngp_check_finite(grads, n,
- * state + 3) on the same stream first; a sum of <= 8 finite fp32 gradients is finite) and travels with the first flag exchange.
- * Same arguments and state layout as ngp_adam_step_fused; a lost peer (timeout) makes the blocks that notice it apply nothing
- * and every later launch a no-op (state[5], sticky). */
 int ngp_adam_step_dp(float* params, float* grads, float* exp_avg, float* exp_avg_sq, void* half_shadow, uint64_t n,
                      uint32_t n_segments, const uint64_t* seg_end, const float* seg_lr, float beta1, float beta2, float eps,
                      float grad_div, float lr_decay_ln, float lr_decay_steps, float growth_factor, float backoff_factor,
@@ -340,8 +332,8 @@ int ngp_adam_step_dp(float* params, float* grads, float* exp_avg, float* exp_avg
                      const uint64_t* peer_grads, const uint64_t* peer_params, const uint64_t* peer_half, const uint64_t* peer_flags,
                      const uint64_t* multicast, void* stream);
 uint64_t ngp_dp_flags_bytes(void);
-/* option 0: timeout of the cross-GPU waits in milliseconds (default 20000); option 1: blocks of the cooperative launch
- * (0 = one per SM). */
+/* option 0: timeout of the cross-GPU waits in milliseconds (default 20000); option 1: blocks of the ngp_adam_step_dp grid
+ * (0 = sized from the slice, the default). */
 int ngp_dp_set_option(int option, int value);
 /* cudaDeviceEnablePeerAccess(peer_device) from the current device (idempotent). */
 int ngp_enable_peer_access(int peer_device);

@@ -428,7 +428,7 @@ def bg_backward(fwd, d_rgb):
 def adam_scaler_step(p, g, m, v, state, seg_end, seg_lr, betas=(0.9, 0.99), eps=1e-15, grad_div=1.0, lr_decay_ln=0.0,
                      lr_decay_steps=0.0, growth=2.0, backoff=0.5, growth_interval=2000):
     """TEST INFRASTRUCTURE - float64 restatement of ONE ``ngp_adam_step`` launch after its finite check (optim.py
-    FusedAdamScaler.step; csrc/train_step.cu adam_step_kernel), i.e. ``scaler.step(optimizer); scaler.update();
+    FusedAdamScaler.step; csrc/adam.cu adam_step_kernel), i.e. ``scaler.step(optimizer); scaler.update();
     optimizer.zero_grad()`` on torch.optim.Adam + LambdaLR + GradScaler over one flat buffer:
 
       found_inf = state[3] or any non-finite g  ->  p, m, v untouched; scale *= backoff, tracker = 0, skipped += 1

@@ -1,16 +1,15 @@
 #!/bin/bash
 # Multi-GPU session: DP correctness (fused peer all-reduce + Adam vs NCCL + Adam) and the bench line for the optimizer-kernel
-# variants.   usage: bash profiles/dp_session_r2.sh <N> <tag> [variants...]   (variants: default pipeline coop coop_pipeline nccl)
+# variants.   usage: bash profiles/dp_session_r2.sh <N> <tag> [variants...]   (variants: default pipeline nccl ...)
 N=${1:-2}
 TAG=${2:-r2}
 shift 2
-VARIANTS=${@:-default pipeline coop}
+VARIANTS=${@:-default pipeline}
 O=gpurun_out
 mkdir -p $O
 RUN="python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29533"
 if [ -z "$SKIP_DP_CHECK" ]; then
 $RUN tests/dp_peer_check.py > $O/dp_check_${TAG}_n$N.json 2> $O/dp_check_${TAG}_n$N.err; echo "dp_check rc $?"; cat $O/dp_check_${TAG}_n$N.json
-NGP_DP_KERNEL=coop $RUN tests/dp_peer_check.py > $O/dp_check_${TAG}_coop_n$N.json 2> $O/dp_check_${TAG}_coop_n$N.err; echo "dp_check coop rc $?"; cat $O/dp_check_${TAG}_coop_n$N.json
 fi
 for v in $VARIANTS; do
   case $v in
@@ -19,8 +18,6 @@ for v in $VARIANTS; do
     no_pipeline) ENVV=""; ARGS="--no-pipeline";;
     skip_check) ENVV=""; ARGS="";;
     pipeline) ENVV=""; ARGS="--pipeline";;
-    coop) ENVV="NGP_DP_KERNEL=coop"; ARGS="";;
-    coop_pipeline) ENVV="NGP_DP_KERNEL=coop"; ARGS="--pipeline";;
     nccl) ENVV=""; ARGS="--nccl";;
     chunks1) ENVV=""; ARGS="--chunks 1";;
     chunks1_pipeline) ENVV=""; ARGS="--chunks 1 --pipeline";;

@@ -69,9 +69,6 @@ SIGNATURES = {
     "ngp_check_finite_fold": (_i32, [_vp, _u64, _vp, _vp, _u64, _vp, _vp]),
     "ngp_adam_step": (_i32, [_vp, _vp, _vp, _vp, _vp, _u64, _u32, C.POINTER(_u64), C.POINTER(_f32), _f32, _f32, _f32, _f32,
                              _f32, _f32, _f32, _f32, _u32, _i32, _vp, _vp, _vp]),
-    "ngp_adam_step_fused": (_i32, [_vp, _vp, _vp, _vp, _vp, _u64, _u32, C.POINTER(_u64), C.POINTER(_f32), _f32, _f32, _f32, _f32,
-                                   _f32, _f32, _f32, _f32, _u32, _i32, _vp, _vp, _u32, _u32, C.POINTER(_u64), C.POINTER(_u64),
-                                   C.POINTER(_u64), C.POINTER(_u64), C.POINTER(_u64), _vp]),
     "ngp_adam_step_dp": (_i32, [_vp, _vp, _vp, _vp, _vp, _u64, _u32, C.POINTER(_u64), C.POINTER(_f32), _f32, _f32, _f32, _f32,
                                 _f32, _f32, _f32, _f32, _u32, _i32, _vp, _vp, _u32, _u32, C.POINTER(_u64), C.POINTER(_u64),
                                 C.POINTER(_u64), C.POINTER(_u64), C.POINTER(_u64), _vp]),

@@ -1,206 +1,17 @@
-// The steps either side of the render inside one `-O` train step (SURVEY.md 8f rows 1 and 2), each as ONE launch
-// instead of the reference's chains of eager elementwise kernels:
+// The small ops at the end of the render inside one `-O` train step (SURVEY.md 8f row 2), each as ONE launch instead of
+// the reference's chains of eager elementwise kernels (the optimizer step after it is csrc/adam.cu):
 //
-//   * ngp_check_finite + ngp_adam_step: GradScaler.unscale_/found_inf + Adam (betas, eps, per-group lr, LambdaLR
-//     decay) + GradScaler.update + refresh of the fp16 shadow of the parameters + zero-fill of the gradient bucket,
-//     over ONE flat fp32 buffer (nerf/utils.py:708-713, main.py:128-131, network_grid.py:170-181).
 //   * ngp_blend_background_forward/backward: `image + (1 - weights_sum) * bg`, the depth normalisation and the
 //     hit mask at the end of run_cuda (nerf/renderer.py:535-557).
 //   * ngp_entropy_loss_forward/backward: the opacity-entropy regulariser of train_step (nerf/utils.py:389-394).
 //
-// All of it is HBM/L2-streaming fp32 work: vectorised, grid sized from the SM count, no tensor cores.
+// All of it is streaming fp32 work, no tensor cores.
 #include <math.h>
 
 #include "common.cuh"
 
 namespace ngp {
 namespace step {
-
-// ---- found_inf -------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) check_finite_kernel(const float4* __restrict__ g4, const float* __restrict__ g,
-                                                           uint64_t n, float* __restrict__ found_inf) {
-    const uint64_t n4 = n / 4;
-    bool bad = false;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (uint64_t)gridDim.x * blockDim.x) {
-        const float4 v = __ldg(g4 + i);
-        // x - x is 0 for finite x and NaN for +-inf / NaN
-        const float s = (v.x - v.x) + (v.y - v.y) + (v.z - v.z) + (v.w - v.w);
-        bad = bad || (s != 0.f);
-    }
-    if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
-        const float v = g[n4 * 4 + threadIdx.x];
-        bad = bad || ((v - v) != 0.f);
-    }
-    if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) *found_inf = 1.0f;
-}
-
-// found_inf of the bucket with the odd-frame twin of the table gradient (ngp_grid_scatter_samples_split) folded in on the
-// way: g[t_lo2 .. t_hi2) += odd, odd = 0 (float2 units; the twin is 8-byte aligned) - one pass over the bucket instead of a
-// fold launch followed by a check launch on the critical path of the data-parallel step
-__global__ void __launch_bounds__(256) check_finite_fold_kernel(float2* __restrict__ g2, uint64_t n2, uint64_t t_lo2, uint64_t t_hi2,
-                                                                float2* __restrict__ odd2, float* __restrict__ found_inf) {
-    bool bad = false;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n2; i += (uint64_t)gridDim.x * blockDim.x) {
-        float2 v = g2[i];
-        if (i >= t_lo2 && i < t_hi2) {
-            const float2 o = odd2[i - t_lo2];
-            if (o.x != 0.f || o.y != 0.f) {
-                v.x += o.x; v.y += o.y;
-                g2[i] = v;
-                odd2[i - t_lo2] = make_float2(0.f, 0.f);
-            }
-        }
-        bad = bad || (((v.x - v.x) + (v.y - v.y)) != 0.f);
-    }
-    if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) *found_inf = 1.0f;
-}
-
-// ---- Adam + GradScaler -------------------------------------------------------------------------------------------
-// state layout (fp32, device): [0] loss scale, [1] growth tracker, [2] optimizer step count, [3] found_inf,
-// [4] steps skipped so far.  `blocks_done` is a zero-initialised uint32 used to elect the last block, which applies
-// GradScaler.update() and bumps the step count after every other block has read the old values.
-struct AdamArgs {
-    float* p;          // parameters (flat fp32)
-    float* g;          // gradients (flat fp32), scaled by state[0]; zero-filled on the way out if zero_grads
-    float* m;          // exp_avg
-    float* v;          // exp_avg_sq
-    __half* h;         // optional fp16 shadow of p
-    uint64_t n;
-    uint32_t n_seg;
-    uint64_t seg_end[NGP_ADAM_MAX_SEGMENTS];  // exclusive end of each lr group in the flat buffer
-    float seg_lr[NGP_ADAM_MAX_SEGMENTS];
-    float beta1, beta2, eps;
-    float grad_div;    // extra divisor for the gradients (data-parallel world size for a mean)
-    float lr_decay_ln; // lr multiplier = exp(lr_decay_ln * min(step, lr_decay_steps))  (LambdaLR 0.1^(it/iters))
-    float lr_decay_steps;
-    float growth, backoff;
-    uint32_t growth_interval;
-    int zero_grads;
-    int deferred;      // 1: a launch that finds state[6] == 0 applies nothing and only raises state[6] (pipelined step, see dp_step.cu)
-    float* state;
-    uint32_t* blocks_done;
-};
-
-__global__ void __launch_bounds__(256) adam_step_kernel(const AdamArgs a) {
-    if (a.deferred && *(volatile float*)(a.state + 6) == 0.f) {
-        // deferred mode, nothing pending yet: every block reads the flag before it signs off, the last one raises it
-        __shared__ bool s_arm_last;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            __threadfence();
-            s_arm_last = atomicAdd(a.blocks_done, 1u) == gridDim.x - 1;
-            if (s_arm_last) { a.state[3] = 0.f; a.state[6] = 1.f; *a.blocks_done = 0u; }
-        }
-        return;
-    }
-    const float scale = a.state[0];
-    const float step0 = a.state[2];
-    const bool skip = a.state[3] != 0.f;
-    const float t = step0 + 1.f;
-    // same expressions as torch's fused Adam (bias corrections evaluated in double, then narrowed) - once per block: two
-    // double-precision pow() per THREAD made this kernel 35 us instead of 23 (13 M instructions, fp64 is slow here)
-    __shared__ float s_coef[3];
-    if (threadIdx.x == 0) {
-        s_coef[0] = (float)(1.0 - pow((double)a.beta1, (double)t));
-        s_coef[1] = (float)sqrt(1.0 - pow((double)a.beta2, (double)t));
-        s_coef[2] = a.lr_decay_ln != 0.f ? expf(a.lr_decay_ln * fminf(step0, a.lr_decay_steps)) : 1.f;
-    }
-    __syncthreads();
-    const float bc1 = s_coef[0], bc2_sqrt = s_coef[1], lr_mult = s_coef[2];
-    const float inv = 1.0f / (scale * a.grad_div);
-    const float w1 = 1.f - a.beta1, w2 = 1.f - a.beta2;
-
-    const uint64_t n4 = a.n / 4;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4 + (a.n & 3 ? 1 : 0);
-         i += (uint64_t)gridDim.x * blockDim.x) {
-        const uint64_t e0 = i * 4;
-        const uint32_t cnt = (uint32_t)((a.n - e0) < 4 ? (a.n - e0) : 4);
-        float g[4], p[4], m[4], v[4];
-        if (cnt == 4) {
-            const float4 g4 = *reinterpret_cast<const float4*>(a.g + e0);
-            g[0] = g4.x; g[1] = g4.y; g[2] = g4.z; g[3] = g4.w;
-        } else {
-            for (uint32_t j = 0; j < 4; ++j) g[j] = j < cnt ? a.g[e0 + j] : 0.f;
-        }
-        if (a.zero_grads) {
-            if (cnt == 4) *reinterpret_cast<float4*>(a.g + e0) = make_float4(0.f, 0.f, 0.f, 0.f);
-            else for (uint32_t j = 0; j < cnt; ++j) a.g[e0 + j] = 0.f;
-        }
-        if (skip) continue;
-        if (cnt == 4) {
-            const float4 p4 = *reinterpret_cast<const float4*>(a.p + e0);
-            const float4 m4 = *reinterpret_cast<const float4*>(a.m + e0);
-            const float4 v4 = *reinterpret_cast<const float4*>(a.v + e0);
-            p[0] = p4.x; p[1] = p4.y; p[2] = p4.z; p[3] = p4.w;
-            m[0] = m4.x; m[1] = m4.y; m[2] = m4.z; m[3] = m4.w;
-            v[0] = v4.x; v[1] = v4.y; v[2] = v4.z; v[3] = v4.w;
-        } else {
-            for (uint32_t j = 0; j < 4; ++j) {
-                p[j] = j < cnt ? a.p[e0 + j] : 0.f; m[j] = j < cnt ? a.m[e0 + j] : 0.f; v[j] = j < cnt ? a.v[e0 + j] : 0.f;
-            }
-        }
-#pragma unroll
-        for (uint32_t j = 0; j < 4; ++j) {
-            // learning-rate group of this element (groups are few and long; segments may split a float4)
-            float lr = a.seg_lr[0];
-#pragma unroll
-            for (uint32_t s = 1; s < NGP_ADAM_MAX_SEGMENTS; ++s)
-                if (s < a.n_seg && e0 + j >= a.seg_end[s - 1]) lr = a.seg_lr[s];
-            const float step_size = lr * lr_mult / bc1;
-            const float gr = g[j] * inv;
-            m[j] = fmaf(w1, gr - m[j], m[j]);                 // exp_avg.lerp_(grad, 1 - beta1)
-            v[j] = a.beta2 * v[j] + w2 * gr * gr;
-            const float denom = sqrtf(v[j]) / bc2_sqrt + a.eps;
-            p[j] -= step_size * m[j] / denom;
-        }
-        if (cnt == 4) {
-            *reinterpret_cast<float4*>(a.p + e0) = make_float4(p[0], p[1], p[2], p[3]);
-            *reinterpret_cast<float4*>(a.m + e0) = make_float4(m[0], m[1], m[2], m[3]);
-            *reinterpret_cast<float4*>(a.v + e0) = make_float4(v[0], v[1], v[2], v[3]);
-            if (a.h) {
-                __half2 h0 = __floats2half2_rn(p[0], p[1]), h1 = __floats2half2_rn(p[2], p[3]);
-                uint2 raw;
-                raw.x = *reinterpret_cast<uint32_t*>(&h0); raw.y = *reinterpret_cast<uint32_t*>(&h1);
-                *reinterpret_cast<uint2*>(a.h + e0) = raw;
-            }
-        } else {
-            for (uint32_t j = 0; j < cnt; ++j) {
-                a.p[e0 + j] = p[j]; a.m[e0 + j] = m[j]; a.v[e0 + j] = v[j];
-                if (a.h) a.h[e0 + j] = __float2half_rn(p[j]);
-            }
-        }
-    }
-
-    // ---- last block: GradScaler.update() + step count (torch/amp/grad_scaler.py: _amp_update_scale_) ----
-    __shared__ bool s_last;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        s_last = atomicAdd(a.blocks_done, 1u) == gridDim.x - 1;
-    }
-    __syncthreads();
-    if (s_last && threadIdx.x == 0) {
-        float tracker = a.state[1];
-        float new_scale = scale;
-        if (skip) {
-            new_scale = scale * a.backoff;
-            tracker = 0.f;
-            a.state[4] += 1.f;
-        } else {
-            a.state[2] = t;
-            tracker += 1.f;
-            if (tracker >= (float)a.growth_interval) {
-                const float grown = scale * a.growth;
-                if (isfinite(grown)) new_scale = grown;
-                tracker = 0.f;
-            }
-        }
-        a.state[0] = new_scale;
-        a.state[1] = tracker;
-        a.state[3] = 0.f;
-        *a.blocks_done = 0u;
-    }
-}
 
 // ---- background blend ---------------------------------------------------------------------------------------------
 // image_out = image + (1 - ws) * bg ; depth_out = clamp(depth - near, 0) / (far - near) ; mask = near < far
@@ -278,59 +89,6 @@ __global__ void __launch_bounds__(256) entropy_backward_kernel(const float* __re
 }  // namespace ngp
 
 using namespace ngp;
-
-extern "C" int ngp_check_finite(const float* grads, uint64_t n, float* found_inf, void* stream) {
-    if (!grads || !found_inf) return NGP_ERR_BAD_ARG;
-    if (n == 0) return NGP_OK;
-    if ((reinterpret_cast<uintptr_t>(grads) & 15) != 0) return NGP_ERR_BAD_ARG;
-    const uint64_t want = (n / 4 + 255) / 256 + 1, cap = (uint64_t)num_sms() * 8;
-    const int blocks = (int)(want < cap ? want : cap);
-    step::check_finite_kernel<<<blocks, 256, 0, as_stream(stream)>>>(reinterpret_cast<const float4*>(grads), grads, n, found_inf);
-    return launch_status();
-}
-
-extern "C" int ngp_check_finite_fold(float* grads, uint64_t n, float* grad_table, float* grad_table_odd, uint64_t table_n,
-                                     float* found_inf, void* stream) {
-    if (!grads || !found_inf || !grad_table || !grad_table_odd) return NGP_ERR_BAD_ARG;
-    if ((n & 1) || (table_n & 1) || grad_table < grads || grad_table + table_n > grads + n) return NGP_ERR_BAD_ARG;
-    if (((reinterpret_cast<uintptr_t>(grads) | reinterpret_cast<uintptr_t>(grad_table) | reinterpret_cast<uintptr_t>(grad_table_odd)) & 7) != 0)
-        return NGP_ERR_BAD_ARG;
-    if (n == 0) return NGP_OK;
-    const uint64_t n2 = n / 2, t_lo2 = (uint64_t)(grad_table - grads) / 2, t_hi2 = t_lo2 + table_n / 2;
-    const uint64_t want = (n2 + 255) / 256, cap = (uint64_t)num_sms() * 8;
-    const int blocks = (int)(want < cap ? want : cap);
-    step::check_finite_fold_kernel<<<blocks, 256, 0, as_stream(stream)>>>(reinterpret_cast<float2*>(grads), n2, t_lo2, t_hi2,
-                                                                         reinterpret_cast<float2*>(grad_table_odd), found_inf);
-    return launch_status();
-}
-
-extern "C" int ngp_adam_step(float* params, float* grads, float* exp_avg, float* exp_avg_sq, void* half_shadow, uint64_t n,
-                             uint32_t n_segments, const uint64_t* seg_end, const float* seg_lr, float beta1, float beta2,
-                             float eps, float grad_div, float lr_decay_ln, float lr_decay_steps, float growth_factor,
-                             float backoff_factor, uint32_t growth_interval, int zero_grads, float* state,
-                             uint32_t* blocks_done, void* stream) {
-    if (!params || !grads || !exp_avg || !exp_avg_sq || !state || !blocks_done || !seg_end || !seg_lr) return NGP_ERR_BAD_ARG;
-    if (n_segments == 0 || n_segments > NGP_ADAM_MAX_SEGMENTS || seg_end[n_segments - 1] != n) return NGP_ERR_BAD_ARG;
-    const uintptr_t al = reinterpret_cast<uintptr_t>(params) | reinterpret_cast<uintptr_t>(grads) |
-                         reinterpret_cast<uintptr_t>(exp_avg) | reinterpret_cast<uintptr_t>(exp_avg_sq);
-    if ((al & 15) != 0 || (reinterpret_cast<uintptr_t>(half_shadow) & 7) != 0) return NGP_ERR_BAD_ARG;
-    if (n == 0) return NGP_OK;
-    step::AdamArgs a;
-    a.p = params; a.g = grads; a.m = exp_avg; a.v = exp_avg_sq; a.h = static_cast<__half*>(half_shadow); a.n = n;
-    a.n_seg = n_segments;
-    for (uint32_t s = 0; s < NGP_ADAM_MAX_SEGMENTS; ++s) {
-        a.seg_end[s] = s < n_segments ? seg_end[s] : n;
-        a.seg_lr[s] = s < n_segments ? seg_lr[s] : 0.f;
-    }
-    a.beta1 = beta1; a.beta2 = beta2; a.eps = eps; a.grad_div = grad_div > 0.f ? grad_div : 1.f;
-    a.lr_decay_ln = lr_decay_ln; a.lr_decay_steps = lr_decay_steps;
-    a.growth = growth_factor; a.backoff = backoff_factor; a.growth_interval = growth_interval;
-    a.zero_grads = zero_grads & 1; a.deferred = (zero_grads >> 1) & 1; a.state = state; a.blocks_done = blocks_done;
-    const uint64_t want = (n / 4 + 255) / 256 + 1, cap = (uint64_t)num_sms() * 8;
-    const int blocks = (int)(want < cap ? want : cap);
-    step::adam_step_kernel<<<blocks, 256, 0, as_stream(stream)>>>(a);
-    return launch_status();
-}
 
 extern "C" int ngp_blend_background_forward(const float* image, const float* weights_sum, const float* depth, const float* bg,
                                             int bg_per_ray, const float* nears, const float* fars, uint32_t N, float* image_out,

@@ -1,4 +1,4 @@
-"""Self-check of the fused peer-memory all-reduce + Adam kernel (csrc/dp_step.cu) against NCCL all_reduce followed by the
+"""Self-check of the fused peer-memory all-reduce + Adam kernel (csrc/adam.cu) against NCCL all_reduce followed by the
 two-launch single-GPU optimizer, on seeded synthetic gradients.  Collective: every rank of the initialised process
 group must call ``run``.  Used by tests/dp_peer_check.py (torchrun script) and by bench.py, which emits the result
 as ``dp_check`` in its JSON line at N > 1 so that every scaling run carries data-parallel correctness evidence.
@@ -46,7 +46,7 @@ def run(device, n=1816256, steps=6, grad_div=1.0):
         ref.flat_grads.copy_(raw * scale)
         torch.cuda.synchronize(device)
         dist.barrier()
-        mine.step_fused()
+        mine.step()
         dist.all_reduce(ref.flat_grads)
         ref.step(zero_grads=True)
         torch.cuda.synchronize(device)

@@ -1,4 +1,4 @@
-"""Adam + GradScaler over ONE flat parameter buffer, one launch per step (csrc/train_step.cu, SURVEY.md 8f-1).
+"""Adam + GradScaler over ONE flat parameter buffer, two launches per step (csrc/adam.cu, SURVEY.md 8f-1).
 
 The reference's optimisation step is ``scaler.step(optimizer); scaler.update()`` on ``torch.optim.Adam(
 model.get_params(lr), betas=(0.9, 0.99), eps=1e-15)`` with a ``LambdaLR(0.1 ** min(iter / iters, 1))`` schedule
@@ -30,8 +30,8 @@ class FusedAdamScaler:
         """param_groups: [{'params': iterable, 'lr': float}, ...] as NeRFNetwork.get_params returns.
         lr_decay: None or (factor, iters) for lr * factor ** min(step / iters, 1).
         peer_memory: a parallel.PeerMemory (data parallel): the gradient bucket, the parameters and their fp16 shadow
-        are then placed in memory that every rank of the group can address, and step_fused() all-reduces the
-        gradients itself over NVLink (csrc/dp_step.cu)."""
+        are then placed in memory that every rank of the group can address, and step() all-reduces the
+        gradients itself over NVLink (csrc/adam.cu)."""
         groups = []
         for g in param_groups:
             ps = [p for p in g["params"] if p.requires_grad]
@@ -66,8 +66,6 @@ class FusedAdamScaler:
         # at 2 ranks (52 vs 64 us) - the multimem instructions cost latency and only pay once the fan-out is large
         env = os.environ.get("NGP_DP_MULTICAST", "auto")
         self.use_multicast = (peer_memory is not None and peer_memory.world > 4) if env == "auto" else env != "0"
-        # "blocks": independent blocks, no grid barriers (default); "coop": the cooperative three-barrier kernel
-        self.dp_kernel = os.environ.get("NGP_DP_KERNEL", "blocks")
         if os.environ.get("NGP_DP_BLOCKS"):
             _cabi.check(_cabi.load().ngp_dp_set_option(1, int(os.environ["NGP_DP_BLOCKS"])), "ngp_dp_set_option")
         if os.environ.get("NGP_DP_TIMEOUT_MS"):
@@ -109,7 +107,7 @@ class FusedAdamScaler:
         # [scale, growth tracker, steps, found_inf, skipped, cross-GPU wait timed out, -, -]
         self.state = torch.tensor([init_scale, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0], device=device, dtype=torch.float32)
         self._blocks_done = torch.zeros(1, device=device, dtype=torch.int32)
-        self._sync = torch.zeros(2, device=device, dtype=torch.int32)  # step_fused: [block election, barrier epoch]
+        self._sync = torch.zeros(2, device=device, dtype=torch.int32)  # ngp_adam_step_dp: [block election, barrier epoch]
 
     # -- layout helpers ------------------------------------------------------------------------------------------
     def attach_grads(self):
@@ -149,6 +147,9 @@ class FusedAdamScaler:
 
     def step(self, zero_grads=True, deferred=False, fold=None):
         """scaler.step(optimizer) + scaler.update() (+ optimizer.zero_grad()): two plain launches, no host sync.
+        ngp_check_finite sets found_inf, then ngp_adam_step applies the update - or, with peer memory, ngp_adam_step_dp
+        all-reduces the gradients itself over NVLink on the way (reduce-scatter by P2P loads, Adam on this rank's slice,
+        new parameters written to every replica; it always zero-fills the gradients).
         deferred: the launch only arms (state[6] = 1) when nothing is pending yet - see TrainStep(pipelined=True).
         fold: optional (grad_table view, odd-frame twin) of the split table scatter, added into the bucket inside the
         finite check."""
@@ -158,44 +159,17 @@ class FusedAdamScaler:
                        _cabi.ptr(fold[1]), fold[0].numel(), self.state[3:].data_ptr())
         else:
             _cabi.call("ngp_check_finite", dev, _cabi.ptr(self.flat_grads), self.numel, self.state[3:].data_ptr())
-        _cabi.call("ngp_adam_step", dev, _cabi.ptr(self.flat_params), _cabi.ptr(self.flat_grads), _cabi.ptr(self.exp_avg),
-                   _cabi.ptr(self.exp_avg_sq), _cabi.ptr(self.flat_half), self.numel, self.n_seg, self.seg_end, self.seg_lr,
-                   float(self.betas[0]), float(self.betas[1]), float(self.eps), self.grad_div, self.lr_decay_ln,
-                   self.lr_decay_steps, float(self.growth_factor), float(self.backoff_factor), int(self.growth_interval),
-                   int(bool(zero_grads)) | (2 if deferred else 0), _cabi.ptr(self.state), _cabi.ptr(self._blocks_done))
-
-    def step_fused(self, deferred=False, fold=None):
-        """The same step as ONE cooperative launch (finite check -> grid barrier -> Adam ...), and - with peer
-        memory - the data-parallel gradient all-reduce fused in: reduce-scatter by P2P loads, Adam on this rank's
-        slice, new parameters written to every replica (csrc/dp_step.cu).  Always zero-fills the gradients.
-        deferred: the launch only arms (state[6] = 1) when nothing is pending yet - see TrainStep(pipelined=True).
-        fold: optional (grad_table view, odd-frame twin) of the split table scatter: the twin is added into the bucket
-        before the update (inside the finite check of the barrier-free data-parallel variant, a launch of its own otherwise)."""
-        dev = self.device
-        if self.peer_ptrs is None:
-            rank, world, pg, pp, ph, pf, mc = 0, 1, None, None, None, None, None
+        args = (_cabi.ptr(self.flat_params), _cabi.ptr(self.flat_grads), _cabi.ptr(self.exp_avg), _cabi.ptr(self.exp_avg_sq),
+                _cabi.ptr(self.flat_half), self.numel, self.n_seg, self.seg_end, self.seg_lr, float(self.betas[0]),
+                float(self.betas[1]), float(self.eps), self.grad_div, self.lr_decay_ln, self.lr_decay_steps,
+                float(self.growth_factor), float(self.backoff_factor), int(self.growth_interval))
+        if self.peer is None or self.peer.world == 1:
+            _cabi.call("ngp_adam_step", dev, *args, int(bool(zero_grads)) | (2 if deferred else 0), _cabi.ptr(self.state),
+                       _cabi.ptr(self._blocks_done))
         else:
-            rank, world = self.peer.rank, self.peer.world
-            pg, pp, ph, pf = self.peer_ptrs
             mc = self.multicast if self.use_multicast else None
-        name = "ngp_adam_step_fused"
-        if world > 1 and self.dp_kernel == "blocks":
-            # barrier-free variant (csrc/dp_step.cu adam_dp_kernel): the inf / nan verdict comes from each rank's own bucket
-            # and rides on the first flag exchange - one small extra launch, no grid barriers, any grid size
-            if fold is not None:
-                _cabi.call("ngp_check_finite_fold", dev, _cabi.ptr(self.flat_grads), self.numel, _cabi.ptr(fold[0]),
-                           _cabi.ptr(fold[1]), fold[0].numel(), self.state[3:].data_ptr())
-                fold = None
-            else:
-                _cabi.call("ngp_check_finite", dev, _cabi.ptr(self.flat_grads), self.numel, self.state[3:].data_ptr())
-            name = "ngp_adam_step_dp"
-        if fold is not None:
-            _cabi.call("ngp_grid_fold_odd", dev, _cabi.ptr(fold[0]), _cabi.ptr(fold[1]), fold[0].numel())
-        _cabi.call(name, dev, _cabi.ptr(self.flat_params), _cabi.ptr(self.flat_grads), _cabi.ptr(self.exp_avg),
-                   _cabi.ptr(self.exp_avg_sq), _cabi.ptr(self.flat_half), self.numel, self.n_seg, self.seg_end, self.seg_lr,
-                   float(self.betas[0]), float(self.betas[1]), float(self.eps), self.grad_div, self.lr_decay_ln,
-                   self.lr_decay_steps, float(self.growth_factor), float(self.backoff_factor), int(self.growth_interval),
-                   int(bool(deferred)), _cabi.ptr(self.state), _cabi.ptr(self._sync), rank, world, pg, pp, ph, pf, mc)
+            _cabi.call("ngp_adam_step_dp", dev, *args, int(bool(deferred)), _cabi.ptr(self.state), _cabi.ptr(self._sync),
+                       self.peer.rank, self.peer.world, *self.peer_ptrs, mc)
 
     def sync_shadow_if_changed(self):
         """Refresh the fp16 shadow if a parameter was edited through torch (load_state_dict, manual init) since the
@@ -229,7 +203,7 @@ class FusedAdamScaler:
 
     @property
     def comm_error(self):
-        """True if a cross-GPU wait inside step_fused() ever timed out (one device->host read)."""
+        """True if a cross-GPU wait inside step() ever timed out (one device->host read)."""
         return bool(self.state[5].item() != 0)
 
     # -- checkpointing (nerf/utils.py:847-968 saves optimizer / scaler state next to the model) ----------------------

@@ -80,7 +80,7 @@ def shard_pixels(H, W, rank, world_size, tile=8):
 
 def owner_slice(numel, rank, world_size):
     """[lo, hi) element range of the flat optimizer buffers that `rank` owns in the fused data-parallel step: the
-    partition csrc/dp_step.cu uses (float4 granularity, ceil(n4 / world) float4s per rank, the tail ranks may own less)."""
+    partition csrc/adam.cu uses (float4 granularity, ceil(n4 / world) float4s per rank, the tail ranks may own less)."""
     n4 = numel // 4
     per = (n4 + world_size - 1) // world_size
     lo = min(per * rank, n4)
@@ -113,7 +113,7 @@ class PeerMemory:
                       NVLS multicast address of the allocation or 0).
     The plumbing is PyTorch's symmetric memory (torch.distributed._symmetric_memory: cuMem allocations whose handles
     are exchanged through the group's store and mapped into every rank); kernels only ever see raw addresses
-    (csrc/dp_step.cu).  Raises RuntimeError when the box cannot do it; callers then fall back to an NCCL all-reduce.
+    (csrc/adam.cu).  Raises RuntimeError when the box cannot do it; callers then fall back to an NCCL all-reduce.
     """
 
     def __init__(self, device, group=None):

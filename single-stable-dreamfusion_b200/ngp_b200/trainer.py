@@ -41,7 +41,7 @@ class TrainStep:
         manual: run the step as the hand-scheduled kernel sequence of _body_manual (no autograd, 13 launches) instead
         of the autograd graph of _body (~58 launches); None = whenever the model has the reference's field shape.
         peer_allreduce: world_size > 1 only - fuse the gradient all-reduce into the optimizer kernel over NVLink peer
-        memory (csrc/dp_step.cu) instead of calling NCCL; None = if peer-addressable memory is available.
+        memory (csrc/adam.cu) instead of calling NCCL; None = if peer-addressable memory is available.
         pipelined (hand-scheduled step only): apply step k's optimizer update (and gradient all-reduce) at the START of
         step k+1, on the side stream, overlapped with that step's ray marching (which reads no parameters).  Same
         arithmetic in the same order; the parameters lag one update behind until flush() - called automatically before
@@ -106,7 +106,7 @@ class TrainStep:
                 self.peer_error = repr(e)
         if fused_optimizer:
             # one flat buffer each for params / grads / moments / fp16 shadow; unscale + Adam + scaler.update + shadow
-            # refresh + zero_grad in one (step_fused) or two (step) launches (optim.py); gradients are SUMMED over ranks
+            # refresh + zero_grad in two launches (optim.py); gradients are SUMMED over ranks
             try:
                 self.opt = FusedAdamScaler(model.get_params(lr), betas=(0.9, 0.99), eps=1e-15, grad_div=1.0,
                                            lr_decay=lr_decay, peer_memory=self.peer)
@@ -140,8 +140,8 @@ class TrainStep:
         # default-priority stream it queued behind the field forward's 592 CTAs whenever both became runnable together
         # (pipelined optimizer: both wait for the update) and delayed the loss kernels by ~25 us - high priority
         self._side_fwd = torch.cuda.Stream(device=device, priority=-1) if self.manual else None
-        # pipelined optimizer launch: its own HIGH-priority stream, so that its 148 cooperative CTAs are placed ahead of the
-        # thousands of ray-marching CTAs it runs beside (otherwise it only starts when the marcher's last wave does)
+        # pipelined optimizer launch: its own HIGH-priority stream, so that its CTAs are placed ahead of the thousands of
+        # ray-marching CTAs it runs beside (otherwise it only starts when the marcher's last wave does)
         self._side_opt = torch.cuda.Stream(device=device, priority=-1) if (self.manual and self.pipelined) else None
         self.mirror_rng = False  # draw (and drop) the randn(3) run_cuda spends on light_d, to keep torch's RNG stream aligned
         # Per-ray march jitter of the hand-scheduled step: drawn by the prologue kernel from a counter-based generator
@@ -157,9 +157,6 @@ class TrainStep:
         # side stream).  Measured: forward 0.488 -> 0.417 ms at 3.3 M samples; 1-2 % of the step at 4096 rays per GPU too
         # (2 and 8 GPUs, bench.py --dp-sweep).  NGP_QUAD_TABLE=0 turns it off.
         self.quad_table = os.environ.get("NGP_QUAD_TABLE", "1") not in ("", "0")
-        # one GPU: finite check (+ odd-frame fold) and Adam as two plain launches instead of the one cooperative launch with
-        # its two grid barriers (NGP_ADAM_KERNEL=coop keeps that one)
-        self.adam_two_launch = os.environ.get("NGP_ADAM_KERNEL", "plain") != "coop"
         self._quads = None
         self.device_noise = bool(self.manual) and os.environ.get("NGP_DEVICE_NOISE", "1") not in ("", "0")
         rank = dist.get_rank() if (world_size > 1 and dist.is_available() and dist.is_initialized()) else 0
@@ -490,7 +487,7 @@ class TrainStep:
         if has_bg:
             main.wait_stream(self._side)
         if g_odd is not None and self.keep_grads:
-            # (otherwise folded by _apply_update, inside or right before the optimizer launch)
+            # (otherwise folded by _apply_update, inside the finite check or right before the NCCL all-reduce)
             _cabi.call("ngp_grid_fold_odd", dev, P(g_table), P(g_odd), g_table.numel())
         if self.keep_grads:
             if self.grad_snapshot is None:
@@ -506,19 +503,13 @@ class TrainStep:
             fold = None
             if self._g_table_odd is not None and not self.keep_grads:
                 fold = (self.opt.grad_view(self.model.encoder.embeddings), self._g_table_odd)
-            two_launch = self.world == 1 and self.adam_two_launch
-            in_check = two_launch or (self.world > 1 and self.opt.peer_ptrs is not None and self.opt.dp_kernel == "blocks")
-            if fold is not None and not in_check:
-                # cooperative kernel / NCCL all-reduce of the bucket: a fold launch of its own, first
-                _cabi.call("ngp_grid_fold_odd", self.device, _cabi.ptr(fold[0]), _cabi.ptr(fold[1]), fold[0].numel())
-                fold = None
             if self.world > 1 and self.opt.peer_ptrs is None:
+                # NCCL all-reduce of the bucket: the twin holds this rank's share only, so it is folded in before the reduce
+                if fold is not None:
+                    _cabi.call("ngp_grid_fold_odd", self.device, _cabi.ptr(fold[0]), _cabi.ptr(fold[1]), fold[0].numel())
+                    fold = None
                 dist.all_reduce(self.opt.flat_grads, op=dist.ReduceOp.SUM)
-            kw = {} if fold is None else {"fold": fold}     # (folded inside the finite check)
-            if two_launch:
-                self.opt.step(deferred=deferred, **kw)      # finite check (+ fold) . Adam: two plain launches
-            else:
-                self.opt.step_fused(deferred=deferred, **kw)
+            self.opt.step(deferred=deferred, fold=fold)
 
     def fold_table_grads(self):
         """Add the odd-frame twin of the table gradient (split scatter) into the bucket now (tests that look at the bucket
@@ -669,7 +660,7 @@ class TrainStep:
             if self.fused_optimizer and self.world > 1 and self.opt.peer_ptrs is not None and self.global_step > 0 \
                     and self._comm_error_lagged():
                 # a cross-GPU wait inside the fused all-reduce + Adam kernel timed out: from that launch on the kernel
-                # applies nothing on any rank that saw the flag (csrc/dp_step.cu) - stop instead of training on
+                # applies nothing on any rank that saw the flag (csrc/adam.cu) - stop instead of training on
                 raise RuntimeError("data-parallel step: a peer did not reach the gradient exchange in time (see "
                                    "NGP_DP_TIMEOUT_MS); parameters were left untouched from that step on")
             if self.use_graph and not self.fused_optimizer:

@@ -1,11 +1,11 @@
 #!/usr/bin/env python
-"""Multi-GPU check of the fused peer-memory all-reduce + Adam kernel (csrc/dp_step.cu).  Run under torchrun:
+"""Multi-GPU check of the fused peer-memory all-reduce + Adam kernel (csrc/adam.cu).  Run under torchrun:
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 \
         tests/dp_peer_check.py [--n 1816256]
 
 Every rank fills its gradient bucket with different seeded values (one step carries an inf on ONE rank), runs
-FusedAdamScaler.step_fused() over peer memory, and compares parameters / fp16 shadow / scaler state with a
+FusedAdamScaler.step() over peer memory, and compares parameters / fp16 shadow / scaler state with a
 single-process reference: NCCL all_reduce of the same buckets followed by the two-launch single-GPU optimizer.
 Also times both variants as CUDA-graph replays.  Rank 0 prints one JSON line; exit code 1 on any mismatch.
 (tests/test_gpu_dp.py launches this when the box has >= 2 GPUs.)
@@ -98,7 +98,7 @@ def main():
         ref.step(zero_grads=True)
 
     try:
-        result["fused_us"] = timed(mine.step_fused) * 1e3
+        result["fused_us"] = timed(mine.step) * 1e3
         result["nccl_plus_adam_us"] = timed(nccl_path) * 1e3
         result["comm_error_after_timing"] = mine.comm_error
         ok = ok and not mine.comm_error

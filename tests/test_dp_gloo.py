@@ -95,7 +95,7 @@ def test_owner_slice_partitions_the_flat_buffer():
 
 
 def _sharded_adam_worker(rank, world, port, out):
-    """Host-side model of csrc/dp_step.cu on CPU tensors: reduce-scatter by reading every rank's bucket, Adam on the owned
+    """Host-side model of csrc/adam.cu on CPU tensors: reduce-scatter by reading every rank's bucket, Adam on the owned
     slice with sharded moments, parameters broadcast from their owner - against single-process Adam on the summed grads."""
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
     dist.init_process_group("gloo", rank=rank, world_size=world)

@@ -1,4 +1,4 @@
-"""GPU tests of the one-launch train-step pieces (csrc/train_step.cu) against the torch ops the reference uses:
+"""GPU tests of the one-launch train-step pieces (csrc/train_step.cu, csrc/adam.cu) against the torch ops the reference uses:
 Adam + GradScaler (main.py:128-131, nerf/utils.py:708-713), the run_cuda tail (nerf/renderer.py:535-557) and the
 entropy regulariser (nerf/utils.py:389-394)."""
 import numpy as np
@@ -17,15 +17,41 @@ def _two_models():
     return a, b
 
 
-@pytest.mark.parametrize("one_launch", [False, True])
-def test_fused_adam_scaler_matches_torch_adam_and_gradscaler(one_launch):
-    """one_launch: the cooperative finite-check + Adam kernel (csrc/dp_step.cu, world 1) instead of the two launches."""
+@pytest.mark.parametrize("layout", ["padded", "unpadded"])
+def test_fused_adam_scaler_matches_torch_adam_and_gradscaler(layout):
+    """padded: FusedAdamScaler.step, whose flat buffers pad every tensor to 8 elements.  unpadded: ngp_check_finite +
+    ngp_adam_step called directly on the same parameters packed back to back - 4373 elements, so the last float4 is
+    partial and the second lr group starts inside a float4 (element 2002)."""
+    import ctypes
+    import math
+    from ngp_b200 import _cabi, field
     from ngp_b200.optim import FusedAdamScaler
-    from ngp_b200 import field
     a, b = _two_models()
     lr = 1e-3
     groups = lambda ps: [{"params": ps[:1], "lr": lr * 10}, {"params": ps[1:], "lr": lr}]  # noqa: E731
-    mine = FusedAdamScaler(groups(a), betas=(0.9, 0.99), eps=1e-15, growth_interval=3, lr_decay=(0.1, 10), grad_div=2.0)
+    if layout == "padded":
+        mine = FusedAdamScaler(groups(a), betas=(0.9, 0.99), eps=1e-15, growth_interval=3, lr_decay=(0.1, 10), grad_div=2.0)
+        state, step, half = mine.state, mine.step, field.cached_half
+    else:
+        flat_p = torch.cat([p.detach().reshape(-1) for p in a])
+        n = flat_p.numel()
+        assert n % 4 == 1 and a[0].numel() % 4 == 2
+        flat_g, m, v, flat_h = torch.zeros_like(flat_p), torch.zeros_like(flat_p), torch.zeros_like(flat_p), flat_p.half()
+        state = torch.tensor([65536.0] + [0.0] * 7, device=DEV)
+        done = torch.zeros(1, dtype=torch.int32, device=DEV)
+        seg_end, seg_lr = (ctypes.c_uint64 * 2)(a[0].numel(), n), (ctypes.c_float * 2)(lr * 10, lr)
+        halves, o = {}, 0
+        for p in a:     # parameters and gradients become views of the flat buffers, as FusedAdamScaler makes them
+            p.data, p.grad = flat_p[o:o + p.numel()].view_as(p), flat_g[o:o + p.numel()].view_as(p)
+            halves[id(p)] = flat_h[o:o + p.numel()].view_as(p)
+            o += p.numel()
+        P = _cabi.ptr
+
+        def step():
+            _cabi.call("ngp_check_finite", DEV, P(flat_g), n, state[3:].data_ptr())
+            _cabi.call("ngp_adam_step", DEV, P(flat_p), P(flat_g), P(m), P(v), P(flat_h), n, 2, seg_end, seg_lr, 0.9, 0.99,
+                       1e-15, 2.0, math.log(0.1) / 10, 10.0, 2.0, 0.5, 3, 1, P(state), P(done))
+        half = lambda p: halves[id(p)]  # noqa: E731
     opt = torch.optim.Adam(groups(b), betas=(0.9, 0.99), eps=1e-15)
     sched = torch.optim.lr_scheduler.LambdaLR(opt, lambda it: 0.1 ** min(it / 10, 1))
     scaler = torch.amp.GradScaler("cuda", growth_interval=3)
@@ -37,12 +63,12 @@ def test_fused_adam_scaler_matches_torch_adam_and_gradscaler(one_launch):
             raw[2][7] = float("inf")            # one overflow step: skipped, scale backs off
         if it == 8:
             raw[0][3, 1] = float("nan")
-        s_mine, s_ref = mine.get_scale(), scaler.get_scale()
+        s_mine, s_ref = state[0].item(), scaler.get_scale()
         assert s_mine == s_ref, (it, s_mine, s_ref)
         for p, q, r in zip(a, b, raw):
             p.grad.copy_(r * s_mine * 2.0)      # "all-reduced sum over 2 ranks" of scaled grads
             q.grad = r * s_ref
-        mine.step_fused() if one_launch else mine.step(zero_grads=True)
+        step()
         scaler.step(opt)
         scaler.update()
         if it not in (5, 8):
@@ -50,9 +76,9 @@ def test_fused_adam_scaler_matches_torch_adam_and_gradscaler(one_launch):
         for p, q in zip(a, b):
             assert torch.isfinite(p).all()
             np.testing.assert_allclose(p.detach().cpu().numpy(), q.detach().cpu().numpy(), rtol=2e-5, atol=1e-7)
-            assert torch.equal(field.cached_half(p), p.detach().half())      # fp16 shadow follows the parameter
+            assert torch.equal(half(p), p.detach().half())                  # fp16 shadow follows the parameter
             assert p.grad.abs().sum().item() == 0                           # zero_grad folded in
-    assert mine.steps_taken == 10 and mine.state[4].item() == 2
+    assert state[2].item() == 10 and state[4].item() == 2
 
 
 def test_fused_adam_params_are_views_and_state_dict_keeps_names():
@@ -203,7 +229,6 @@ def test_hand_scheduled_step_matches_autograd_step(views, n_chunks):
             _g.append(_s.opt.flat_grads.clone())
             _s.opt.flat_grads.zero_()
         step.opt.step = capture
-        step.opt.step_fused = capture
         torch.manual_seed(5)
         loss = step(ro, rd, G)
         torch.cuda.synchronize()
@@ -222,7 +247,7 @@ def test_hand_scheduled_step_matches_autograd_step(views, n_chunks):
 
 
 def test_hand_scheduled_step_graph_replay_and_packed_inputs():
-    """Graph replays of the hand-scheduled step (cooperative optimizer kernel + side-stream branch inside the graph)
+    """Graph replays of the hand-scheduled step (optimizer launches + side-stream branch inside the graph)
     follow the eager step; packed inputs reach the static buffers with one copy."""
     from ngp_b200 import provider
     from ngp_b200.trainer import TrainStep

@@ -35,9 +35,8 @@ CONFIGS = {
     "graph": dict(kw=dict(graph=True, device_rays=(HW, 0, 1)), env={}, grad_steps=(0, 1, 2, 7, 15, 16, 19)),
     # the schedule of the multi-GPU default: step k's update runs at the start of step k + 1
     "graph_pipelined": dict(kw=dict(graph=True, device_rays=(HW, 0, 1), pipelined=True), env={}, grad_steps=(0, 16, 19)),
-    # the cooperative finite-check + Adam kernel with its own fold launch, and a LambdaLR decay that saturates at step 10
-    "graph_coop_lr_decay": dict(kw=dict(graph=True, device_rays=(HW, 0, 1), lr_decay=(0.1, 10)),
-                                env={"NGP_ADAM_KERNEL": "coop"}, grad_steps=(0, 16, 19)),
+    # bench.py's one-GPU step with a LambdaLR decay that saturates at step 10
+    "graph_lr_decay": dict(kw=dict(graph=True, device_rays=(HW, 0, 1), lr_decay=(0.1, 10)), env={}, grad_steps=(0, 16, 19)),
     # eager, host rays, the fallback kernels: per-level gathers, one-buffer scatter, ray-ordered marcher
     "eager_fallbacks": dict(kw=dict(graph=False), env={"NGP_QUAD_TABLE": "0", "NGP_SPLIT_SCATTER": "0", "NGP_PACKED_MARCH": "0"},
                             grad_steps=(0, 16, 19)),
