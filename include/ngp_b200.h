@@ -353,7 +353,12 @@ int ngp_enable_peer_access(int peer_device);
  * of n_rays_total (0 = N); all per-ray pointers are the chunk's.  Outputs: weights_sum[N], depth[N], image[N,3] (before the
  * blend), grad_bg[N,3] (optional), grad_sigmas[M], grad_rgbs[M,3]; *loss += the chunk's share of the entropy loss.
  * bg_half: f16[N,3] or NULL (then the colour bg_const).  Optional bookkeeping when counter != NULL (atomic):
- * *samples_total += counter[0]; step_counter[*cur_row] += counter. */
+ * *samples_total += counter[0]; step_counter[*cur_row] += counter.
+ * ngp_train_light: the light direction of a shaded train step (nerf/renderer.py:461-464), one thread:
+ * light f32[6] = (safe_normalize(rays_o[0..2] + z), z) with z three N(0, 1) draws (Box-Muller) from the generator of rng
+ * (u64[3], as above) at keys no ray's jitter uses.  advance = 0: call it after a prologue launch that drew noise (it takes
+ * that launch's counter, rng[1] - 1); advance = 1: it takes rng[1] and advances the counter itself.  So the light is
+ * reproducible for a given (seed, step) and fresh on every step, graph replays included. */
 int ngp_train_prologue(const float* rays_o, const float* rays_d, const float* aabb, uint32_t N, float min_near, float* nears,
                        float* fars, int* counters, uint32_t n_counters, float* loss, int* step_counter, int* local_step,
                        int* cur_row, float* noises, uint64_t* rng, void* stream);
@@ -363,20 +368,43 @@ int ngp_train_ray_loss(const float* sigmas, const float* rgbs, const float* delt
                        float* depth, float* image, float* grad_bg, float* grad_sigmas, float* grad_rgbs, float* loss,
                        const int* counter, unsigned long long* samples_total, int* step_counter, const int* cur_row,
                        void* stream);
+int ngp_train_light(const float* rays_o, uint64_t* rng, int advance, float* light, void* stream);
 
 /* Shading path as a 7-point stencil (nerf/network_grid.py:90-144; csrc/shading.cu).  ngp_stencil_points: xyzs f32[M,3] ->
  * out f32[M*K,3], K = 7 (x, x+eps e_x, x-eps e_x, x+eps e_y, ...) or 6 (with_centre == 0), shifted points clamped to
- * [-bound, bound] (:93-98): the K points of a sample are K consecutive rows of ONE field batch.  ngp_shade_forward: the K
+ * [-bound, bound] (:93-98): the K points of a sample are K consecutive rows of ONE field batch.  count_ptr (optional, as
+ * ngp_field_forward takes it): M is then the capacity and min(*count_ptr, M) samples are read on the device; count_out
+ * (optional) receives K times that count, for the field kernels that follow (K * M must fit an int).  NULL / NULL: all M.
+ * ngp_shade_forward: the K
  * densities (sigma_all f32[M*K]) -> normal f32[M,3] = safe_normalize(-0.5 (s+ - s-) / eps), NaN -> 0 (:100-114) and, for
  * K = 7 and color_out != NULL, the colour of mode 0 lambertian (albedo * (ratio + (1 - ratio) max(n.l, 0)), albedo = the
  * centre row of rgb_all f32[M*K,3]), 1 textureless, 2 normal ((n + 1) / 2) with autocast's half roundings (:126-140).
  * ngp_shade_backward: d_normal f32[M,3] and / or d_color f32[M,3] -> d_sigma_all f32[M*K] (0 for the centre row) and
  * d_rgb_all f32[M*K,3] (centre row only; may be NULL). */
-int ngp_stencil_points(const float* xyzs, uint32_t M, float eps, float bound, int with_centre, float* out, void* stream);
+int ngp_stencil_points(const float* xyzs, uint32_t M, const int* count_ptr, float eps, float bound, int with_centre, float* out,
+                       int* count_out, void* stream);
 int ngp_shade_forward(const float* sigma_all, const float* rgb_all, uint32_t M, uint32_t K, const float* light, float ratio, int mode,
                       float* normal_out, float* color_out, void* stream);
 int ngp_shade_backward(const float* sigma_all, const float* rgb_all, uint32_t M, uint32_t K, const float* light, float ratio, int mode,
                        const float* d_normal, const float* d_color, float* d_sigma_all, float* d_rgb_all, void* stream);
+/* The same pair for the hand-scheduled shaded train step (K = 7, the sample count M = min(*count_ptr, M_cap) read on the
+ * device, light f32[3] in device memory).  Rows >= M of every output are left untouched.
+ * ngp_shade_forward_step: sigma_all f32[7 M_cap] / rgb_all f32[7 M_cap,3] -> sigma f32[M_cap] (the centre row's density)
+ * and rgb f32[M_cap,3] (the colour of ngp_shade_forward, same arithmetic): the per-sample rows ngp_train_ray_loss reads.
+ * ngp_shade_backward_step: the composite gradients d_sigma f32[M_cap] / d_rgb f32[M_cap,3] (ngp_train_ray_loss) ->
+ * d_sigma_all f32[7 M_cap] (centre row: d_sigma; the six stencil rows: the normal's gradient) and d_rgb_all f32[7 M_cap,3]
+ * (centre row: d(albedo) in mode 0, else 0; the stencil rows 0), with the orientation regulariser of
+ * nerf/renderer.py:485-486 fused in: loss_orient = (1 - exp(-sigma)).detach() * clamp(n . d, 0)^2 (dirs f32[M_cap,3]: the
+ * per-sample ray directions), averaged over the step's samples - the sum of counters[2c], c < n_counters, the i32[n,2]
+ * counters of every ray chain of the step, so all their marches must be complete - and *loss += lambda_orient * mean (one
+ * atomic per block).  Its gradient is multiplied by *scale (the GradScaler scale; NULL = 1) and joins the normal's
+ * gradient ahead of the colour's.  loss may be NULL. */
+int ngp_shade_forward_step(const float* sigma_all, const float* rgb_all, uint32_t M_cap, const int* count_ptr, const float* light,
+                           float ratio, int mode, float* sigma, float* rgb, void* stream);
+int ngp_shade_backward_step(const float* sigma_all, const float* rgb_all, uint32_t M_cap, const int* count_ptr, const int* counters,
+                            uint32_t n_counters, const float* dirs, const float* light, float ratio, int mode, const float* d_sigma,
+                            const float* d_rgb, float lambda_orient, const float* scale, float* d_sigma_all, float* d_rgb_all,
+                            float* loss, void* stream);
 
 /* The inference branch of run_cuda (nerf/renderer.py:496-532) as ONE launch: the reference's host loop - count alive rays
  * (a device->host sync per iteration), n_step = clamp(N / n_alive, 1, 8), march_rays, field, composite_rays, mask-compact -

@@ -76,9 +76,13 @@ SIGNATURES = {
     "ngp_dp_set_option": (_i32, [_i32, _i32]),
     "ngp_enable_peer_access": (_i32, [_i32]),
     "ngp_train_prologue": (_i32, [_vp, _vp, _vp, _u32, _f32, _vp, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "ngp_stencil_points": (_i32, [_vp, _u32, _f32, _f32, _i32, _vp, _vp]),
+    "ngp_train_light": (_i32, [_vp, _vp, _i32, _vp, _vp]),
+    "ngp_stencil_points": (_i32, [_vp, _u32, _vp, _f32, _f32, _i32, _vp, _vp, _vp]),
     "ngp_shade_forward": (_i32, [_vp, _vp, _u32, _u32, _vp, _f32, _i32, _vp, _vp, _vp]),
     "ngp_shade_backward": (_i32, [_vp, _vp, _u32, _u32, _vp, _f32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "ngp_shade_forward_step": (_i32, [_vp, _vp, _u32, _vp, _vp, _f32, _i32, _vp, _vp, _vp]),
+    "ngp_shade_backward_step": (_i32, [_vp, _vp, _u32, _vp, _vp, _u32, _vp, _vp, _f32, _i32, _vp, _vp, _f32, _vp, _vp, _vp, _vp,
+                                       _vp]),
     "ngp_render_infer_workspace": (_u64, [_u32]),
     "ngp_render_infer_loop": (_i32, [_vp, _vp, _vp, _vp, _u32, _f32, _f32, _u32, _u32, _u32, _vp, _f32, _vp, _vp, _vp, _u32, _u32, _f32,
                                      _u32, _u32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _u32, _u32, _vp, _vp, _vp, _vp, _u64, _vp]),

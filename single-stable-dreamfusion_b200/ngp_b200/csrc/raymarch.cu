@@ -513,6 +513,36 @@ __global__ void train_prologue_rays_kernel(const RayGen g, float* __restrict__ r
     if (noises && threadIdx.x == 0) rng_step_done(rng, s_rng[1]);
 }
 
+// Light direction of a shaded train step (nerf/renderer.py:461-464): light_d = safe_normalize(rays_o[0] + randn(3)), with
+// the three normal draws taken from the same counter-based generator as the march jitter, on keys no ray uses: ray_noise at
+// "ray" indices 2^32 - 1 ... 2^32 - 4 (four uniforms -> two Box-Muller pairs, three of the four normals used).  One thread.
+// advance == 0: a prologue launch of this step drew the jitter and advanced the counter, so the step's counter is rng[1] - 1;
+// advance == 1: no jitter was drawn, the step's counter is rng[1] and this launch advances it.
+__global__ void train_light_kernel(const float* __restrict__ rays_o, unsigned long long* rng, int advance, float* __restrict__ light) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    const unsigned long long seed = rng[0], ctr = advance ? rng[1] : rng[1] - 1ull;
+    float u[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) u[j] = ray_noise(seed, ctr, 0xFFFFFFFFu - (uint32_t)j);
+    // 1 - u lies in [2^-24, 1]: the logarithm is finite
+    const float r0 = sqrtf(-2.0f * logf(1.0f - u[0])), r1 = sqrtf(-2.0f * logf(1.0f - u[2]));
+    float s0, c0, s1, c1;
+    sincospif(2.0f * u[1], &s0, &c0);
+    sincospif(2.0f * u[3], &s1, &c1);
+    const float z[3] = {r0 * c0, r0 * s0, r1 * c1};
+    float x[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) x[a] = __fadd_rn(rays_o[a], z[a]);
+    const float nn = __fadd_rn(__fadd_rn(__fmul_rn(x[0], x[0]), __fmul_rn(x[1], x[1])), __fmul_rn(x[2], x[2]));
+    const float nrm = sqrtf(fmaxf(nn, 1e-20f));
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        light[a] = __fdiv_rn(x[a], nrm);
+        light[3 + a] = z[a];
+    }
+    if (advance) rng[1] = ctr + 1ull;
+}
+
 __global__ void sph_from_ray_kernel(const float* __restrict__ rays_o, const float* __restrict__ rays_d, float radius,
                                     uint32_t N, float* coords) {
     const uint32_t n = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1893,6 +1923,12 @@ extern "C" int ngp_train_prologue_rays(const float* poses, const float* intrinsi
     march::train_prologue_rays_kernel<<<cdiv(N, 128), 128, 0, as_stream(stream)>>>(
         g, rays_o, rays_d, aabb, min_near, nears, fars, counters, n_counters, loss, step_counter, local_step, cur_row, noises,
         reinterpret_cast<unsigned long long*>(rng));
+    return launch_status();
+}
+
+extern "C" int ngp_train_light(const float* rays_o, uint64_t* rng, int advance, float* light, void* stream) {
+    if (!rays_o || !rng || !light) return NGP_ERR_BAD_ARG;
+    march::train_light_kernel<<<1, 32, 0, as_stream(stream)>>>(rays_o, reinterpret_cast<unsigned long long*>(rng), advance, light);
     return launch_status();
 }
 

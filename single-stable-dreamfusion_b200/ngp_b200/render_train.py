@@ -16,12 +16,33 @@ from . import _cabi
 from .field import cached_half
 
 _BYTES_PER_ROW = 12 + 8 + 4 + 12 + 64 + 128 + 128 + 4 + 12 + 64  # xyzs deltas sigma rgb enc h1 h2 d_sigma d_rgb d_enc
+# Shaded steps of the hand-scheduled train step (trainer.py) also keep the 7 stencil rows of every sample (centre + six
+# shifted points, csrc/shading.cu) and the per-sample ray direction (orientation regulariser):
+#   extra bytes = 7 * cap * _STENCIL_BYTES_PER_ROW + 12 * cap,   cap = round_up(n_rays * max_steps, 128)
+# e.g. one 64x64 view (4096 rays) at max_steps 1024: cap = 4 194 304 rows -> 12.6 GB of stencil rows (+ 50 MB of directions)
+# on top of cap * _BYTES_PER_ROW = 1.8 GB of per-sample rows; 8 views: about 100 GB.
+_STENCIL_BYTES_PER_ROW = 12 + 4 + 12 + 64 + 128 + 128 + 4 + 12 + 64  # xyzs sigma rgb enc h1 h2 d_sigma d_rgb d_enc
+
+
+class StencilRows:
+    """The field batch of a shaded step: 7 rows per sample (ngp_stencil_points), with the field's saved activations and
+    gradients; counter[0] = 7 x the chain's sample count, written on the device by ngp_stencil_points."""
+
+    def __init__(self, cap, device):
+        rows = 7 * cap
+        f32, f16 = torch.float32, torch.half
+        e = lambda *shape, dtype=f32: torch.empty(*shape, device=device, dtype=dtype)  # noqa: E731
+        self.cap = rows
+        self.xyzs, self.sigma, self.rgb = e(rows, 3), e(rows), e(rows, 3)
+        self.enc, self.h1, self.h2 = e(rows, 32, dtype=f16), e(rows, 64, dtype=f16), e(rows, 64, dtype=f16)
+        self.d_sigma, self.d_rgb, self.d_enc = e(rows), e(rows, 3), e(rows, 32, dtype=f16)
+        self.counter = torch.zeros(2, device=device, dtype=torch.int32)
 
 
 class TrainWorkspace:
     """Static per-(N, max_steps) buffers of the training render."""
 
-    def __init__(self, n_rays, max_steps, device, counter=None):
+    def __init__(self, n_rays, max_steps, device, counter=None, shaded=False):
         # always the worst case (every ray emits max_steps samples): the marcher can then never overflow, so no ray is
         # ever dropped and rows >= counter[0] are never read
         cap = n_rays * max_steps
@@ -37,6 +58,9 @@ class TrainWorkspace:
         self._device = device
         self._march_ws = None
         self.counter = torch.zeros(2, device=device, dtype=torch.int32) if counter is None else counter
+        # shaded steps: per-sample ray directions (written by the marcher) and the stencil rows
+        self.dirs = e(cap, 3) if shaded else None
+        self.stencil = StencilRows(cap, device) if shaded else None
 
     @property
     def march_ws(self):
@@ -51,7 +75,8 @@ class TrainWorkspace:
 
     @property
     def nbytes(self):
-        return self.cap * _BYTES_PER_ROW
+        extra = 0 if self.stencil is None else 7 * self.cap * _STENCIL_BYTES_PER_ROW + 12 * self.cap
+        return self.cap * _BYTES_PER_ROW + extra
 
 
 class _RenderTrain(Function):

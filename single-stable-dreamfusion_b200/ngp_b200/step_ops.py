@@ -146,7 +146,8 @@ def stencil_points(x, eps, bound, with_centre=True):
     M = x.shape[0]
     K = 7 if with_centre else 6
     out = torch.empty(M * K, 3, device=x.device, dtype=torch.float32)
-    _cabi.call("ngp_stencil_points", x.device, _cabi.ptr(x), M, float(eps), float(bound), int(with_centre), _cabi.ptr(out))
+    _cabi.call("ngp_stencil_points", x.device, _cabi.ptr(x), M, None, float(eps), float(bound), int(with_centre), _cabi.ptr(out),
+               None)
     return out
 
 

@@ -40,6 +40,12 @@ class TrainStep:
         (this TrainStep's H of them) of every view on the device (nerf/utils.py:43-106 get_rays; hand-scheduled step only).
         manual: run the step as the hand-scheduled kernel sequence of _body_manual (no autograd, 13 launches) instead
         of the autograd graph of _body (~58 launches); None = whenever the model has the reference's field shape.
+        shading: 'albedo' (default), or 'lambertian' / 'textureless' / 'normal' for every step of this TrainStep (the
+        reference draws these after albedo_iters with ambient_ratio 0.1 and adds lambda_orient * loss_orient,
+        nerf/utils.py:345-356,396-398).  Shaded steps run hand-scheduled too - stencil, field forward over 7 rows per sample,
+        shade, per-ray loss, shade backward with the orientation term, field backward, scatter (_manual_compute) - when
+        world_size == 1, overlap is off and lambda_smooth == 0; otherwise (and with manual=False) through the autograd
+        step.  manual=True with one of those settings raises.
         peer_allreduce: world_size > 1 only - fuse the gradient all-reduce into the optimizer kernel over NVLink peer
         memory (csrc/adam.cu) instead of calling NCCL; None = if peer-addressable memory is available.
         pipelined (hand-scheduled step only): apply step k's optimizer update (and gradient all-reduce) at the START of
@@ -50,15 +56,25 @@ class TrainStep:
         rank hide behind the marcher), off on one GPU (the update is 1.6 % of the step and the marcher is issue-bound)."""
         self.model, self.H, self.W = model, H, W
         # shading != 'albedo' (after albedo_iters the reference draws 'textureless' / 'lambertian' with ambient_ratio 0.1,
-        # nerf/utils.py:345-356, and adds lambda_orient * loss_orient [+ lambda_smooth * loss_smooth], :396-402): runs
-        # through the autograd step (the 7-point stencil kernels of csrc/shading.cu under run_cuda)
+        # nerf/utils.py:345-356, and adds lambda_orient * loss_orient [+ lambda_smooth * loss_smooth], :396-402): the
+        # hand-scheduled step over the 7-point stencil kernels of csrc/shading.cu; the settings it does not cover take the
+        # autograd step (the same kernels under run_cuda)
+        from .step_ops import SHADING_MODES
         self.shading = shading
         self.ambient_ratio = (1.0 if shading == "albedo" else 0.1) if ambient_ratio is None else float(ambient_ratio)
         self.lambda_orient, self.lambda_smooth = float(lambda_orient), float(lambda_smooth)
+        self._shade_mode = None     # hand-scheduled shaded step: csrc/shading.cu mode (0 lambertian, 1 textureless, 2 normal)
         if shading != "albedo":
-            if manual:
-                raise RuntimeError("the hand-scheduled step implements albedo shading; use manual=False for shaded steps")
-            manual = False
+            unsupported = [name for name, bad in (("shading=%r" % (shading,), shading not in SHADING_MODES),
+                                                  ("lambda_smooth > 0", self.lambda_smooth > 0),
+                                                  ("world_size > 1", world_size > 1), ("overlap=True", bool(overlap))) if bad]
+            if unsupported:
+                if manual:
+                    raise RuntimeError("the hand-scheduled shaded step does not support %s; use manual=False"
+                                       % ", ".join(unsupported))
+                manual = False
+            elif manual is None or manual:
+                self._shade_mode = SHADING_MODES[shading]
         # overlap (hand-scheduled, graphed step only): the ray-marching half of step k+1 (prologue + march: it reads rays and
         # the occupancy bitfield, no parameters) runs on its own stream WHILE the field / loss / backward / optimizer half of
         # step k runs - two CUDA graphs per step and two alternating workspace sets, ordered by ordinary stream events.
@@ -79,6 +95,7 @@ class TrainStep:
         # entropy term is a MEAN over all rays of the job, so each rank's local mean is weighted 1 / world.
         self.lam_local = float(lambda_entropy) / float(world_size)
         self.fixed_noises = None  # tests: per-ray perturbation noise [N] used instead of a fresh torch.rand draw
+        self.fixed_light = None   # tests: light direction [3] of a shaded hand-scheduled step instead of a fresh draw
         # table-gradient scatter into two buffers (even / odd row pairs both as 16-byte reds); NGP_SPLIT_SCATTER=0: one buffer
         self.split_scatter = os.environ.get("NGP_SPLIT_SCATTER", "1") not in ("", "0")
         self._g_table_odd = None
@@ -93,6 +110,8 @@ class TrainStep:
         self.device = device
         self.fused_optimizer = fused_optimizer
         self.manual = bool(fused_optimizer and self._manual_supported()) if manual is None else bool(manual)
+        if not self.manual:
+            self._shade_mode = None
         if self.manual and not (fused_optimizer and self._manual_supported()):
             raise RuntimeError("the hand-scheduled step needs the fused optimizer and the reference's field / bg-net shapes")
         if self.device_rays is not None and not self.manual:
@@ -143,7 +162,10 @@ class TrainStep:
         # pipelined optimizer launch: its own HIGH-priority stream, so that its CTAs are placed ahead of the thousands of
         # ray-marching CTAs it runs beside (otherwise it only starts when the marcher's last wave does)
         self._side_opt = torch.cuda.Stream(device=device, priority=-1) if (self.manual and self.pipelined) else None
-        self.mirror_rng = False  # draw (and drop) the randn(3) run_cuda spends on light_d, to keep torch's RNG stream aligned
+        # draw the randn(3) run_cuda spends on light_d (and drop it under albedo shading), to keep torch's RNG stream aligned;
+        # shaded steps then take their light from it as run_cuda does.  Otherwise a shaded step draws its light on the
+        # device (ngp_train_light: same generator as the march jitter below).
+        self.mirror_rng = False
         # Per-ray march jitter of the hand-scheduled step: drawn by the prologue kernel from a counter-based generator
         # (csrc/raymarch.cu ray_noise; [seed, step counter, scratch]) instead of a torch.rand launch - in graph mode torch
         # also enqueues two seed / offset fill kernels before every replay of a graph that holds one of its generators.
@@ -240,10 +262,16 @@ class TrainStep:
         n_chunks = self.n_chunks if self.n_chunks else 2
         n_chunks = max(1, min(int(n_chunks), N // 128 if N >= 256 else 1))
         e = lambda *shape, dtype=torch.float32: torch.empty(*shape, device=dev, dtype=dtype)  # noqa: E731
+        shaded = self._shade_mode is not None
         m = dict(N=N, nears=e(N), fars=e(N), noises=e(N), weights_sum=e(N), depth=e(N), image=e(N, 3),
                  bg=e(N, 3, dtype=torch.half), d_bg=e(N, 3), loss=torch.zeros((), device=dev),
                  counters=torch.zeros(n_chunks, 2, dtype=torch.int32, device=dev),
                  cur_row=torch.zeros(1, dtype=torch.int32, device=dev), chunks=[])
+        if shaded:
+            # the step's light (direction, then the three normal draws behind it; ngp_train_light) - one for all chains -
+            # and, with several chains, one event per chain's march: the orientation mean runs over the samples of all
+            m["light"] = torch.zeros(6, device=dev)
+            m["march_done"] = [torch.cuda.Event() for _ in range(n_chunks)] if n_chunks > 1 else []
         base = 0
         sizes = [N // n_chunks + (1 if c < N % n_chunks else 0) for c in range(n_chunks)]
         fr = os.environ.get("NGP_CHUNK_FRACTIONS")    # e.g. "0.4,0.6": unequal chains (their kernel phases then interleave)
@@ -253,7 +281,7 @@ class TrainStep:
             sizes[-1] = N - sum(sizes[:-1])
         for c in range(n_chunks):
             n_c = sizes[c]
-            ws = TrainWorkspace(n_c, self.max_steps, dev, counter=m["counters"][c])
+            ws = TrainWorkspace(n_c, self.max_steps, dev, counter=m["counters"][c], shaded=shaded)
             m["chunks"].append((base, n_c, ws))
             base += n_c
         self.model._train_ws = m["chunks"][0][2]  # (what run_cuda's own fused path would allocate; kept for introspection)
@@ -273,6 +301,10 @@ class TrainStep:
 
             prologue (near/far, counters, bookkeeping) . rand . { march x3 . field fwd . ray loss (composite fwd + blend +
             both loss gradients + composite bwd) . field bwd . grid scatter } . all-reduce + Adam + GradScaler
+
+        Shaded steps (shading != 'albedo'): light (ngp_train_light) after the prologue, the marcher also writes per-sample
+        directions, and each chain runs  stencil (7 rows per sample) . field fwd (7 M rows) . shade fwd (centre density +
+        colour into the per-sample rows) . ray loss . shade bwd (+ orientation term) . field bwd (7 M) . grid scatter.
 
         with the background net on a side stream (forward beside the marching, backward beside the field backward).
         The braces run as TWO chains over the two halves of the rays on parallel streams: the marcher and the per-ray
@@ -382,8 +414,19 @@ class TrainStep:
                 if self.pipelined:
                     self._side_fwd.wait_stream(self._side_opt)
                 self._bg_forward(m, c, main)    # (reads the generated ray directions)
+        shaded = self._shade_mode is not None
         if self.mirror_rng:
-            torch.randn(3, device=dev)  # nerf/renderer.py:464 (light direction; unused by albedo shading)
+            z = torch.randn(3, device=dev)  # nerf/renderer.py:464 (light direction; unused by albedo shading)
+            if shaded and self.fixed_light is None:
+                from .renderer import safe_normalize
+                m["light"][:3].copy_(safe_normalize(ro[0] + z))      # run_cuda's own expression
+                m["light"][3:].copy_(z)
+        if shaded:
+            if self.fixed_light is not None:
+                m["light"][:3].copy_(self.fixed_light)
+            elif not self.mirror_rng:
+                # after the prologue: rays_o[0] may be a generated ray; advance the counter unless the prologue did
+                _cabi.call("ngp_train_light", dev, P(ro), P(self._rng), 0 if dev_noise else 1, P(m["light"]))
         if self.fixed_noises is not None:
             m["noises"].copy_(self.fixed_noises)
         elif not dev_noise:
@@ -394,20 +437,23 @@ class TrainStep:
         streams = [main] + chain[:len(chunks) - 1]
         for st in streams[1:]:
             st.wait_stream(main)
-        for st, (base, n_c, ws) in zip(streams, chunks):
+        for k, (st, (base, n_c, ws)) in enumerate(zip(streams, chunks)):
             with torch.cuda.stream(st):
                 sl = slice(base, base + n_c)
+                dirs = P(ws.dirs) if ws.dirs is not None else None     # (shaded steps: the orientation term reads them)
                 if self.packed_march and self.max_steps <= 2048:
                     # one launch, no scratch: rows claimed with the reference's atomicAdd, rays land in completion order
                     _cabi.call("ngp_march_rays_train_packed", dev, P(ro[sl]), P(rd[sl]), P(model.density_bitfield),
                                float(model.bound), 0.0, int(self.max_steps), n_c, int(model.cascade), int(model.grid_size),
-                               ws.cap, P(m["nears"][sl]), P(m["fars"][sl]), P(ws.xyzs), None, P(ws.deltas), P(ws.rays),
+                               ws.cap, P(m["nears"][sl]), P(m["fars"][sl]), P(ws.xyzs), dirs, P(ws.deltas), P(ws.rays),
                                P(ws.counter), P(m["noises"][sl]))
                 else:
                     _cabi.call("ngp_march_rays_train", dev, P(ro[sl]), P(rd[sl]), P(model.density_bitfield), float(model.bound),
                                0.0, int(self.max_steps), n_c, int(model.cascade), int(model.grid_size), ws.cap,
-                               P(m["nears"][sl]), P(m["fars"][sl]), P(ws.xyzs), None, P(ws.deltas), P(ws.rays), P(ws.counter),
+                               P(m["nears"][sl]), P(m["fars"][sl]), P(ws.xyzs), dirs, P(ws.deltas), P(ws.rays), P(ws.counter),
                                P(m["noises"][sl]), P(ws.march_ws), ws.march_ws.numel())
+                if m.get("march_done"):
+                    m["march_done"][k].record(st)
         if which is not None:       # a phase of its own: join the chains (in the fused step they run on into phase 2)
             for st in streams[1:]:
                 main.wait_stream(st)
@@ -435,20 +481,31 @@ class TrainStep:
             for st in streams[1:]:
                 st.wait_stream(main)
 
+        shade = self._shade_mode
+        ratio = float(self.ambient_ratio)
+
         def forward_and_loss(base, n_c, ws):
             sl = slice(base, base + n_c)
+            # shaded: the field runs on the 7 stencil rows of every sample (count 7 M written on the device)
+            rows = ws if shade is None else ws.stencil
+            if shade is not None:
+                _cabi.call("ngp_stencil_points", dev, P(ws.xyzs), ws.cap, P(ws.counter), 1e-2, float(model.bound), 1, P(rows.xyzs),
+                           P(rows.counter))
             if self.pipelined:
                 torch.cuda.current_stream(dev).wait_stream(self._side_opt)  # the field reads the updated parameters
             if c["quads"] is not None:
                 torch.cuda.current_stream(dev).wait_stream(self._side_fwd)   # the step's quad table
-                _cabi.call("ngp_field_forward_quads", dev, P(ws.xyzs), ws.cap, P(ws.counter), P(table_h), P(c["quads"]),
+                _cabi.call("ngp_field_forward_quads", dev, P(rows.xyzs), rows.cap, P(rows.counter), P(table_h), P(c["quads"]),
                            P(enc.offsets), L, 2, S, int(enc.base_resolution), int(enc.gridtype_id), int(bool(enc.align_corners)),
-                           float(model.bound), *[P(t) for t in hw_field], 64, 4, P(ws.sigma), P(ws.rgb), P(ws.enc), P(ws.h1),
-                           P(ws.h2))
+                           float(model.bound), *[P(t) for t in hw_field], 64, 4, P(rows.sigma), P(rows.rgb), P(rows.enc),
+                           P(rows.h1), P(rows.h2))
             else:
-                _cabi.call("ngp_field_forward", dev, P(ws.xyzs), ws.cap, P(ws.counter), P(table_h), P(enc.offsets), L, 2, S,
+                _cabi.call("ngp_field_forward", dev, P(rows.xyzs), rows.cap, P(rows.counter), P(table_h), P(enc.offsets), L, 2, S,
                            int(enc.base_resolution), int(enc.gridtype_id), int(bool(enc.align_corners)), float(model.bound),
-                           *[P(t) for t in hw_field], 64, 4, P(ws.sigma), P(ws.rgb), P(ws.enc), P(ws.h1), P(ws.h2))
+                           *[P(t) for t in hw_field], 64, 4, P(rows.sigma), P(rows.rgb), P(rows.enc), P(rows.h1), P(rows.h2))
+            if shade is not None:   # centre density + shaded colour into the ordinary per-sample rows
+                _cabi.call("ngp_shade_forward_step", dev, P(rows.sigma), P(rows.rgb), ws.cap, P(ws.counter), P(m["light"]), ratio,
+                           shade, P(ws.sigma), P(ws.rgb))
             if has_bg:
                 torch.cuda.current_stream(dev).wait_stream(self._side_fwd)
             _cabi.call("ngp_train_ray_loss", dev, P(ws.sigma), P(ws.rgb), P(ws.deltas), P(ws.rays), ws.cap, n_c, 1e-4,
@@ -458,16 +515,24 @@ class TrainStep:
                        P(m["cur_row"]))
 
         def backward(ws):
-            _cabi.call("ngp_field_backward", dev, ws.cap, P(ws.counter), P(hw_field[0]), P(hw_field[2]), P(hw_field[4]), 64, 4,
-                       P(ws.d_sigma), P(ws.d_rgb), P(ws.sigma), P(ws.rgb), P(ws.enc), P(ws.h1), P(ws.h2), P(ws.d_enc),
-                       *[P(t) for t in g_field])
+            rows = ws if shade is None else ws.stencil
+            if shade is not None:
+                for ev in m["march_done"]:      # the orientation mean needs every chain's sample count
+                    torch.cuda.current_stream(dev).wait_event(ev)
+                _cabi.call("ngp_shade_backward_step", dev, P(rows.sigma), P(rows.rgb), ws.cap, P(ws.counter), P(m["counters"]),
+                           len(chunks), P(ws.dirs), P(m["light"]), ratio, shade, P(ws.d_sigma), P(ws.d_rgb),
+                           float(self.lambda_orient) / self.world, opt.state.data_ptr(), P(rows.d_sigma), P(rows.d_rgb),
+                           P(m["loss"]))
+            _cabi.call("ngp_field_backward", dev, rows.cap, P(rows.counter), P(hw_field[0]), P(hw_field[2]), P(hw_field[4]), 64, 4,
+                       P(rows.d_sigma), P(rows.d_rgb), P(rows.sigma), P(rows.rgb), P(rows.enc), P(rows.h1), P(rows.h2),
+                       P(rows.d_enc), *[P(t) for t in g_field])
             if g_odd is None:
-                _cabi.call("ngp_grid_scatter_samples", dev, P(ws.d_enc), P(ws.xyzs), float(model.bound), P(ws.counter), ws.cap,
-                           P(enc.offsets), L, 2, S, int(enc.base_resolution), int(enc.gridtype_id), int(bool(enc.align_corners)),
-                           P(g_table))
+                _cabi.call("ngp_grid_scatter_samples", dev, P(rows.d_enc), P(rows.xyzs), float(model.bound), P(rows.counter),
+                           rows.cap, P(enc.offsets), L, 2, S, int(enc.base_resolution), int(enc.gridtype_id),
+                           int(bool(enc.align_corners)), P(g_table))
             else:
-                _cabi.call("ngp_grid_scatter_samples_split", dev, P(ws.d_enc), P(ws.xyzs), float(model.bound), P(ws.counter),
-                           ws.cap, P(enc.offsets), L, 2, S, int(enc.base_resolution), int(enc.gridtype_id),
+                _cabi.call("ngp_grid_scatter_samples_split", dev, P(rows.d_enc), P(rows.xyzs), float(model.bound), P(rows.counter),
+                           rows.cap, P(enc.offsets), L, 2, S, int(enc.base_resolution), int(enc.gridtype_id),
                            int(bool(enc.align_corners)), P(g_table), P(g_odd))
 
         for st, (base, n_c, ws) in zip(streams, chunks):
